@@ -24,6 +24,8 @@ data-path collective: "weak" scaling); `value` is the whole-job aggregate.  The 
                 sources) on all host cores, bounded sample
 
 `--impl reference` times that CPU implementation instead (bench.py's only other use of oracle/).
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) to DIR/output.npy (see dump_outputs), so that
+two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -47,6 +49,7 @@ BYTES_PER_FRAME = 236  # I/O 16 + reverb rings 192 + echo 12 + chorus 16 (SURVEY
 CFG3_OPS_PER_FRAME = 266  # dry 2 + flanger 26 + ring modulator 60 + distortion 147 + compressor 31 (DESIGN.md section 5)
 METRIC = "channel-samples/s, 4-slot EAX reverb chain @48 kHz"
 UNIT = "channel-samples/s"
+DUMP_BYTES = 32 << 20  # --dump-outputs: at most this much of the output (the cfg4 block is 512 MB)
 
 
 def workload_config(streams):
@@ -58,6 +61,20 @@ def workload_config(streams):
         "l2": "per-step working set (>10 GB of delay lines + 1 GB of I/O) exceeds the 126 MB L2; no flush needed",
         "parallelism": "streams sharded per GPU, no data-path collective",
     }
+
+
+def dump_outputs(directory, np, torch, y):
+    """Write y ([stream][frame][channel] fp32, what the caller of oalsfx_engine_mix receives) as DIR/output.npy: every
+    stream when the block fits in DUMP_BYTES, else a fixed sample of streams (the same for every run with the same
+    stream count), whose indices go to DIR/output_streams.npy (float64)."""
+    streams = y.shape[0]
+    keep = min(streams, DUMP_BYTES // (y[0].numel() * y.element_size()))
+    index = np.arange(streams)
+    if keep < streams:
+        index = np.sort(np.random.default_rng(0).choice(streams, keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "output.npy"), y[torch.from_numpy(index).to(y.device)].cpu().numpy())
+    np.save(os.path.join(directory, "output_streams.npy"), index.astype(np.float64))
 
 
 # ---- CPU reference leg (test infrastructure under oracle/) ------------------------------------------
@@ -72,10 +89,7 @@ def _load_cpu_reference():
                 [ctypes.c_uint32, ctypes.POINTER(ctypes.c_double)]
             lib.orc_bench.restype = ctypes.c_double
             return kind, lib
-    if os.path.isdir("/root/reference/src") or os.path.exists(os.path.join(ROOT, "oracle", "oalsfx_oracle.cpp")):
-        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "all"], check=False)
-        return _load_cpu_reference() if os.path.exists(os.path.join(ROOT, "oracle/_build/liboalsfx_oracle.so")) else (None, None)
-    return None, None
+    return None, None  # build() makes oracle/_build; the tree is not written to from here
 
 
 def cpu_run(lib, threads, streams, blocks):
@@ -311,7 +325,11 @@ def main():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--skip-configs", action="store_true", help="leave out the cfg1 / cfg2 / cfg3 records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step (a fixed sample of at most 32 MB of it) to DIR/output.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -377,6 +395,8 @@ def main():
     total_ms_max = float(t.item())
     value = world * S * C * F * args.steps / (total_ms_max * 1e-3)
     assert bool(torch.isfinite(y).all()), "non-finite output"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, np, torch, y)  # before the legs below overwrite y
 
     # -- the all-streams output bus (BASELINE config 4) at full size: oalsfx_engine_mix_bus = mix + one deterministic pass
     #    over the block's output + (N > 1) one NCCL all-reduce of the [frames][channels] bus over NVLink.

@@ -36,9 +36,11 @@ def test_restatement_matches_golden(case):
 
 
 def test_reference_matches_golden(ref):
+    """The golden hashes and the POD sizes test_abi.py pins (108 / 112 bytes) are what the compiled reference gives."""
     for name, fmt, rate, effect_count, script, x in QUICK:
         y = H.run_script_orc(ref, fmt, rate, effect_count, script, x)
         assert np.array_equal(_sha(y), GOLDEN["sha256/" + name]), name
+    assert ref.orc_sizeof_effect_props() == 108 and ref.orc_sizeof_effect() == 112
 
 
 def test_restatement_matches_reference_on_full_matrix(ref):
@@ -61,10 +63,11 @@ def test_restatement_ten_seconds_chain(ref):
     assert np.array_equal(a, b)
 
 
-def test_noise_generators_agree(ref):
-    """The hash noise is identical in numpy (tests), the reference shim and the restatement."""
+def test_noise_generators_agree():
+    """The hash noise is identical in numpy (tests), the C shim the reference is wrapped with (oracle/ref_shim.cpp,
+    here compiled against include/oalsfxpp.h) and the restatement."""
     want = H.noise(5, 2, 1000, first_frame=123)
-    for lib in (ref, H.oracle_lib()):
+    for lib in (H.api_shim("emu"), H.oracle_lib()):
         got = np.zeros((1000, 2), np.float32)
         lib.orc_noise(H.SEED, 5, 2, 123, 1000, got.ctypes.data)
         assert np.array_equal(want, got)
