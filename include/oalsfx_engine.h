@@ -179,6 +179,26 @@ const char* oalsfx_reverb_preset_name(int index);
 long long oalsfx_plan_placement(const int32_t* class_of_stream, int n_streams, int32_t* engine_index_of_stream,
 	int32_t* class_triples, int class_capacity, int* class_count);
 
+/* Stream placement inside the engine.  In OALSFX_PLACEMENT_AUTO mode the engine keeps every 32-stream tile class-pure
+ * by itself: before a block whose configuration changed (set_effect, set_sends, a consumed update) it moves streams
+ * between its internal lanes -- a stream already in a pure tile of its own settings stays where it is, so changing k
+ * streams moves about k streams -- growing its arenas by whole tiles when needed (they never shrink).  Caller stream
+ * indices and every buffer keep their meaning and layout: set_effect, set_sends, mix, mix_bus, reduce_bus,
+ * debug_state, snapshot and restore take and return caller streams; the mix permutes the block into lane order and
+ * back on the device (two extra passes over the block).  A snapshot is written in caller stream order, so it restores
+ * into an engine in either mode.  Only speed, launch_count, last_kernel and device_bytes show the placement; host
+ * buffers take the unsliced staging path.  Switching back to OALSFX_PLACEMENT_CALLER (the default: lane = stream)
+ * moves every stream back to its own lane, after which the engine runs as one that was never placed.  Returns
+ * OALSFX_OK or OALSFX_ERR_ARGUMENT for an unknown mode; a failed move reports OALSFX_ERR_DEVICE.  Synchronizes. */
+enum {
+	OALSFX_PLACEMENT_CALLER = 0, /* default: engine lane of stream s is s */
+	OALSFX_PLACEMENT_AUTO = 1    /* the engine moves streams between lanes so that every tile holds one class */
+};
+int oalsfx_engine_set_placement(oalsfx_engine* e, int mode);
+/* lane_of_stream[s] for s < n (n <= num_streams, lane_of_stream may be NULL when n == 0): the engine lane that holds
+ * caller stream s now.  Returns the engine's lane count (a multiple of 32) or a negative OALSFX_ERR_* code. */
+long long oalsfx_engine_lanes(oalsfx_engine* e, int32_t* lane_of_stream, int n);
+
 /* Library build identification, e.g. "oalsfx_b200 sm_100a cuda". */
 const char* oalsfx_build_info(void);
 

@@ -13,6 +13,7 @@
 #include <string>
 
 #include "mix.cuh"
+#include "place.cuh"
 
 namespace oalsfx {
 
@@ -39,6 +40,31 @@ public:
 	// `tiles` is a HOST array.
 	virtual bool zero_lanes(uint32_t* base, long long tile_stride, int words, const TileRef* tiles, int n_tiles,
 		void* stream) = 0;
+	// Stream placement (place.cuh).  Arenas are tile-major, base[tile * tile_stride + word * 32 + lane]; lane lists are
+	// DEVICE arrays.  copy_lanes: for every entry i, dst lane to[i] words [dst_w0, +words) = src lane from[i] words
+	// [src_w0, +words); from[i] < 0 writes zeros, to[i] < 0 skips the entry, a null list is the identity (lane i).
+	// gather_io: dst (TILED, `frames` frames, lane_tiles tiles) lane l = caller stream stream_of_lane[l] of src
+	// (src[(s/32)*ts + (s%32)*ls + f*fs + c*cs]), zeros where stream_of_lane[l] < 0.  scatter_io: the reverse, caller
+	// rows only.  These defaults are place.cuh's host loops over the kernels' element bodies and need device memory the
+	// host can address: the CPU test backend's.  cuda_backend.cu overrides all three with the sm_100a kernels.
+	virtual bool copy_lanes(uint32_t* dst, long long dst_ts, int dst_w0, const uint32_t* src, long long src_ts, int src_w0,
+		int words, const int32_t* from, const int32_t* to, int n, void*)
+	{
+		place::copy_lanes_host(dst, dst_ts, dst_w0, src, src_ts, src_w0, words, from, to, n);
+		return true;
+	}
+	virtual bool gather_io(const float* src, long long ts, long long ls, long long fs, long long cs, const int32_t* stream_of_lane,
+		int lane_tiles, int frames, int channels, float* dst, void*)
+	{
+		place::gather_io_host(src, ts, ls, fs, cs, stream_of_lane, lane_tiles, frames, channels, dst);
+		return true;
+	}
+	virtual bool scatter_io(const float* src, const int32_t* stream_of_lane, int lane_tiles, int frames, int channels, float* dst,
+		long long ts, long long ls, long long fs, long long cs, void*)
+	{
+		place::scatter_io_host(src, stream_of_lane, lane_tiles, frames, channels, dst, ts, ls, fs, cs);
+		return true;
+	}
 	virtual bool launch_mix(int kernel_id, const MixArgs& args, void* stream) = 0;
 	// The relay kernels (relay.cuh) are device-only code: the CPU test backend answers false and the engine
 	// keeps such groups on the single-effect passes.

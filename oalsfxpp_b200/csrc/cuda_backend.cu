@@ -378,6 +378,30 @@ public:
 		return check(cudaStreamSynchronize(st), "cudaStreamSynchronize") && ok;
 	}
 
+	bool copy_lanes(uint32_t* dst, long long dst_ts, int dst_w0, const uint32_t* src, long long src_ts, int src_w0, int words,
+		const int32_t* from, const int32_t* to, int n, void* stream) override
+	{
+		DeviceScope scope(this);
+		return scope.ok && launch_copy_lanes(dst, dst_ts, dst_w0, src, src_ts, src_w0, words, from, to, n, static_cast<cudaStream_t>(stream)) &&
+			check(cudaGetLastError(), "copy_lanes_kernel");
+	}
+
+	bool gather_io(const float* src, long long ts, long long ls, long long fs, long long cs, const int32_t* stream_of_lane,
+		int lane_tiles, int frames, int channels, float* dst, void* stream) override
+	{
+		DeviceScope scope(this);
+		return scope.ok && launch_gather_io(src, ts, ls, fs, cs, stream_of_lane, lane_tiles, frames, channels, dst,
+			static_cast<cudaStream_t>(stream)) && check(cudaGetLastError(), "gather_io_kernel");
+	}
+
+	bool scatter_io(const float* src, const int32_t* stream_of_lane, int lane_tiles, int frames, int channels, float* dst,
+		long long ts, long long ls, long long fs, long long cs, void* stream) override
+	{
+		DeviceScope scope(this);
+		return scope.ok && launch_scatter_io(src, stream_of_lane, lane_tiles, frames, channels, dst, ts, ls, fs, cs,
+			static_cast<cudaStream_t>(stream)) && check(cudaGetLastError(), "scatter_io_kernel");
+	}
+
 	bool launch_mix(int kernel_id, const MixArgs& args, void* stream) override
 	{
 		DeviceScope scope(this);

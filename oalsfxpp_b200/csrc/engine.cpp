@@ -68,6 +68,8 @@ struct Group {
 	bool multi = false;        // class-per-tile launch: every tile has ONE parameter class, coefficient blocks per tile from HBM
 	size_t tile_begin = 0;     // into the concatenated tile list
 	int tile_count = 0;
+	int multi_kernel = -1;     // class-per-tile launch: its kernel and slot kinds
+	int multi_kinds[kMaxSlots] = {};
 };
 
 } // namespace
@@ -78,7 +80,7 @@ struct oalsfx_engine {
 	Backend* be = nullptr;
 	int streams = 0, tiles = 0, channels = 0, slots = 0;
 
-	// per-stream configuration (host)
+	// per-lane configuration (host): lane = caller stream unless the engine places its streams (placed)
 	std::vector<int> fx_class[kMaxSlots];
 	std::vector<int> send_class;
 	std::vector<uint8_t> pending;       // bit s: slot s has an un-consumed `update`
@@ -133,6 +135,29 @@ struct oalsfx_engine {
 	size_t send_table_cap = 0;
 	int32_t* lane_class_dev[kMaxSlots] = {};
 	int32_t* lane_send_dev = nullptr;
+
+	// Stream placement (oalsfx_engine_set_placement).  `tiles` stays the caller's ceil(streams / 32); the arenas hold
+	// arena_tiles >= tiles (only AUTO placement grows them).  While `placed`, the configuration vectors above are indexed
+	// by lane (arena_tiles * 32 entries) and lane_of_stream / stream_of_lane (-1: padding lane) map caller streams.
+	int placement = OALSFX_PLACEMENT_CALLER;
+	bool placed = false;
+	bool place_oom = false;             // the last placement could not grow the arenas (nothing was changed)
+	int arena_tiles = 0;
+	std::vector<int32_t> lane_of_stream, stream_of_lane;
+	std::vector<GroupKey> tile_key;     // per arena tile: the key its caller streams share
+	std::vector<uint8_t> tile_active;   // per arena tile: holds a caller stream
+	bool refill_padding = true;         // every padding lane gets its tile-mate's state at the next placement
+	int32_t* stream_of_lane_dev = nullptr;
+	size_t stream_of_lane_cap = 0;
+	int32_t* lane_list_dev = nullptr;   // lane lists of copy_lanes
+	size_t lane_list_cap = 0;
+	uint32_t* move_scratch = nullptr;   // bounded staging arena of the lane moves and of snapshot / restore
+	size_t move_scratch_cap = 0;        // words
+	float* io_in = nullptr;             // one block of the mix in lane order (TILED)
+	float* io_out = nullptr;
+	size_t io_cap = 0;                  // floats each
+	int lane_count() const { return placed ? arena_tiles * kLanes : streams; }
+	int lane_of(int s) const { return placed ? lane_of_stream[static_cast<size_t>(s)] : s; }
 
 	std::vector<Group> groups;
 	// Class-per-tile launch (duo_multi_kernel): the class table and every tile's class index in HBM; `groups` is
@@ -230,6 +255,11 @@ struct oalsfx_engine {
 		}
 		be->release(stage_in);
 		be->release(stage_out);
+		be->release(stream_of_lane_dev);
+		be->release(lane_list_dev);
+		be->release(move_scratch);
+		be->release(io_in);
+		be->release(io_out);
 		be->stream_destroy(pipe_in);
 		be->stream_destroy(pipe_run);
 		be->stream_destroy(pipe_out);
@@ -437,17 +467,17 @@ struct oalsfx_engine {
 			return true;
 		}
 		const size_t new_tile_bytes = static_cast<size_t>(words) * kLanes * sizeof(float);
-		float* fresh = static_cast<float*>(dev_alloc(new_tile_bytes * static_cast<size_t>(tiles)));
+		float* fresh = static_cast<float*>(dev_alloc(new_tile_bytes * static_cast<size_t>(arena_tiles)));
 		if (!fresh) {
 			return false;
 		}
 		if (ring[slot]) {
 			const size_t old_tile_bytes = static_cast<size_t>(ring_cap[slot]) * kLanes * sizeof(float);
 			if (!be->copy_2d(fresh, new_tile_bytes, ring[slot], old_tile_bytes, old_tile_bytes,
-					static_cast<size_t>(tiles), nullptr) || !be->sync(nullptr)) {
+					static_cast<size_t>(arena_tiles), nullptr) || !be->sync(nullptr)) {
 				return false;
 			}
-			device_bytes -= static_cast<long long>(old_tile_bytes) * tiles;
+			device_bytes -= static_cast<long long>(old_tile_bytes) * arena_tiles;
 			be->release(ring[slot]);
 		}
 		ring[slot] = fresh;
@@ -512,7 +542,7 @@ struct oalsfx_engine {
 				sends[i * kSendCount + 1 + static_cast<size_t>(k)] = send_classes[i].aux_coef[k];
 			}
 		}
-		const size_t padded = static_cast<size_t>(tiles) * kLanes;
+		const size_t padded = static_cast<size_t>(arena_tiles) * kLanes;
 		if (!grow(slot_table_dev, slot_table_cap, coefs.size()) || !grow(send_table_dev, send_table_cap, sends.size())) {
 			return false;
 		}
@@ -527,13 +557,13 @@ struct oalsfx_engine {
 		bool ok = be->upload(slot_table_dev, coefs.data(), coefs.size() * sizeof(SlotCoef), nullptr) &&
 			be->upload(send_table_dev, sends.data(), sends.size() * sizeof(SendCoef), nullptr);
 		std::vector<int32_t> idx(padded, 0);
-		for (int s = 0; s < streams; ++s) {
+		for (int s = 0; s < lane_count(); ++s) {
 			idx[static_cast<size_t>(s)] = send_class[static_cast<size_t>(s)];
 		}
 		ok = ok && be->upload(lane_send_dev, idx.data(), padded * sizeof(int32_t), nullptr) && be->sync(nullptr);
 		for (int k = 0; k < kMaxSlots && ok; ++k) {
 			std::fill(idx.begin(), idx.end(), 0);
-			for (int s = 0; s < streams; ++s) {
+			for (int s = 0; s < lane_count(); ++s) {
 				idx[static_cast<size_t>(s)] = fx_class[k][static_cast<size_t>(s)];
 			}
 			ok = be->upload(lane_class_dev[k], idx.data(), padded * sizeof(int32_t), nullptr) && be->sync(nullptr);
@@ -548,6 +578,9 @@ struct oalsfx_engine {
 			compact_classes();
 		}
 		quiesce();  // the group tables below are uploaded in place
+		if (placed) {
+			return place_streams() && build_placed_groups();
+		}
 		groups.clear();
 		const GroupKey k0 = key_of(0);
 		bool uniform = true;
@@ -657,14 +690,8 @@ struct oalsfx_engine {
 		int active = 0;
 		for (const auto& kv : by_key) {
 			const GroupKey& key = kv.first;
-			const SendClass& sc = send_classes[static_cast<size_t>(key.send)];
-			bool ok = sc.direct_coef.filter_type == 0;
 			int kinds[kMaxSlots];
-			for (int s = 0; s < kMaxSlots; ++s) {
-				const FxClass& fc = classes[static_cast<size_t>(key.fx[s])];
-				kinds[s] = kind_of_type(fc.type);
-				ok = ok && (kinds[s] == kKindNull || sc.aux_coef[s].filter_type == 0) && !(fc.coef.flags & kCoefUnstable);
-			}
+			bool ok = multi_kinds_of(key, kinds);
 			if (first) {
 				std::memcpy(multi_kinds, kinds, sizeof(kinds));
 				chain = channels == 2 && std::memcmp(infos[kChainStereo].kind, kinds, sizeof(kinds)) == 0;
@@ -684,30 +711,14 @@ struct oalsfx_engine {
 			if (!ok) {
 				return true;
 			}
-			Group g;
-			g.key = key;
-			MixArgs a;
-			fill_common(a, g, 2, nullptr, nullptr, OALSFX_LAYOUT_STREAM_MAJOR, 2, 0);
-			MixClassEntry e;
-			std::memset(&e, 0, sizeof(e));
-			int pos = 0;
-			for (int s = 0; s < kMaxSlots; ++s) { // the chain kernel addresses slots by index, the relay by compacted position
-				if (chain || kinds[s] != kKindNull) {
-					fill_slot(a, g, pos, s, false);
-					e.pending |= ((key.pending >> s) & 1U) << pos;
-					++pos;
-				}
-			}
-			sanitize_gains(a);
-			std::memcpy(e.coefs, reinterpret_cast<const char*>(&a) + kMixCoefOffset, kMixCoefBytes);
-			table.push_back(e);
+			table.push_back(multi_entry(key, kinds, chain));
 			pending_any |= key.pending;
 		}
 		if (!grow(class_table_dev, class_table_cap, table.size())) {
 			return false;
 		}
 		if (!tile_class_dev) {
-			tile_class_dev = static_cast<int32_t*>(dev_alloc(static_cast<size_t>(tiles) * sizeof(int32_t)));
+			tile_class_dev = static_cast<int32_t*>(dev_alloc(static_cast<size_t>(arena_tiles) * sizeof(int32_t)));
 			if (!tile_class_dev) {
 				return false;
 			}
@@ -725,8 +736,646 @@ struct oalsfx_engine {
 		g.identity = true;
 		g.multi = true;
 		g.tile_count = tiles;
+		g.multi_kernel = multi_kernel;
+		std::memcpy(g.multi_kinds, multi_kinds, sizeof(multi_kinds));
 		groups.assign(1, g);
 		return true;
+	}
+
+	// ---- stream placement (OALSFX_PLACEMENT_AUTO) ----------------------------------------------------------
+	// Every arena is tile-major, base[tile * words * 32 + word * 32 + lane]: the rings of each slot, its state, the send state.
+	struct Arena { uint32_t* base; int words; };
+	std::vector<Arena> arenas(bool with_rings) const
+	{
+		std::vector<Arena> out;
+		for (int s = 0; s < slots; ++s) {
+			if (with_rings && ring_cap[s] > 0) {
+				out.push_back(Arena{reinterpret_cast<uint32_t*>(ring[s]), ring_cap[s]});
+			}
+			out.push_back(Arena{slot_state[s], kSlotStateWords});
+		}
+		out.push_back(Arena{send_state, kSendStateWords});
+		return out;
+	}
+
+	static constexpr size_t kMoveScratchWords = size_t(64) << 20; // 256 MB: the lane moves and snapshots go through it in chunks
+
+	bool ensure_scratch(size_t words)
+	{
+		if (words <= move_scratch_cap) {
+			return true;
+		}
+		be->sync(nullptr);
+		if (move_scratch) {
+			device_bytes -= static_cast<long long>(move_scratch_cap * sizeof(uint32_t));
+			be->release(move_scratch);
+		}
+		move_scratch_cap = words;
+		move_scratch = static_cast<uint32_t*>(dev_alloc(words * sizeof(uint32_t)));
+		if (!move_scratch) {
+			move_scratch_cap = 0;
+		}
+		return move_scratch != nullptr;
+	}
+
+	bool upload_lane_list(const std::vector<int32_t>& v)
+	{
+		return grow(lane_list_dev, lane_list_cap, v.size()) &&
+			be->upload(lane_list_dev, v.data(), v.size() * sizeof(int32_t), nullptr) && be->sync(nullptr);
+	}
+
+	// Moves the contents of lane `first` to lane `second` in every arena, in place (the moving lanes may swap): per chunk
+	// of words, a gather of the sources (in source-lane order) into the scratch arena, then a scatter sorted by destination.
+	bool move_lanes(const std::vector<std::pair<int32_t, int32_t>>& moves)
+	{
+		if (moves.empty()) {
+			return true;
+		}
+		const size_t n = moves.size();
+		std::vector<std::pair<int32_t, int32_t>> by_src(moves);
+		std::sort(by_src.begin(), by_src.end());
+		std::vector<std::pair<int32_t, int32_t>> by_dst(n);   // (destination lane, scratch position)
+		for (size_t p = 0; p < n; ++p) {
+			by_dst[p] = std::make_pair(by_src[p].second, static_cast<int32_t>(p));
+		}
+		std::sort(by_dst.begin(), by_dst.end());
+		std::vector<int32_t> lists(3 * n);
+		for (size_t i = 0; i < n; ++i) {
+			lists[i] = by_src[i].first;
+			lists[n + i] = by_dst[i].first;
+			lists[2 * n + i] = by_dst[i].second;
+		}
+		if (!upload_lane_list(lists)) {
+			return false;
+		}
+		const int32_t* src_lanes = lane_list_dev;
+		const int32_t* dst_lanes = lane_list_dev + n;
+		const int32_t* scratch_pos = lane_list_dev + 2 * n;
+		const size_t rows = (n + kLanes - 1) / kLanes * kLanes;
+		bool ok = true;
+		for (const Arena& a : arenas(true)) {
+			const int cw = static_cast<int>(std::max<size_t>(1, std::min<size_t>(static_cast<size_t>(a.words), kMoveScratchWords / rows)));
+			ok = ok && ensure_scratch(rows * static_cast<size_t>(cw));
+			const long long ts = static_cast<long long>(a.words) * kLanes;
+			for (int w0 = 0; w0 < a.words && ok; w0 += cw) {
+				const int nw = std::min(cw, a.words - w0);
+				const long long sts = static_cast<long long>(nw) * kLanes;
+				ok = be->copy_lanes(move_scratch, sts, 0, a.base, ts, w0, nw, src_lanes, nullptr, static_cast<int>(n), nullptr) &&
+					be->copy_lanes(a.base, ts, w0, move_scratch, sts, 0, nw, scratch_pos, dst_lanes, static_cast<int>(n), nullptr);
+			}
+		}
+		return ok && be->sync(nullptr);
+	}
+
+	// More tiles in every arena: the new buffers are allocated first, so a failure leaves the engine as it was.  Rings
+	// are tile-major: the old contents are one prefix of the new buffer.
+	bool grow_arena(int new_tiles)
+	{
+		struct Resize { void** p; size_t tile_bytes; void* fresh; };
+		std::vector<Resize> list;
+		for (int s = 0; s < slots; ++s) {
+			if (ring[s]) {
+				list.push_back(Resize{reinterpret_cast<void**>(&ring[s]), static_cast<size_t>(ring_cap[s]) * kLanes * sizeof(float), nullptr});
+			}
+			list.push_back(Resize{reinterpret_cast<void**>(&slot_state[s]), static_cast<size_t>(kSlotStateWords) * kLanes * sizeof(uint32_t), nullptr});
+		}
+		list.push_back(Resize{reinterpret_cast<void**>(&send_state), static_cast<size_t>(kSendStateWords) * kLanes * sizeof(uint32_t), nullptr});
+		if (tile_class_dev) {
+			list.push_back(Resize{reinterpret_cast<void**>(&tile_class_dev), sizeof(int32_t), nullptr});
+		}
+		for (Resize& r : list) {
+			r.fresh = dev_alloc(r.tile_bytes * static_cast<size_t>(new_tiles));
+			if (!r.fresh) {
+				for (Resize& q : list) {
+					if (q.fresh) {
+						be->release(q.fresh);
+						device_bytes -= static_cast<long long>(q.tile_bytes) * new_tiles;
+					}
+				}
+				return false;
+			}
+		}
+		bool ok = true;
+		for (Resize& r : list) {
+			ok = ok && be->copy_2d(r.fresh, r.tile_bytes, *r.p, r.tile_bytes, r.tile_bytes, static_cast<size_t>(arena_tiles), nullptr);
+		}
+		ok = ok && be->sync(nullptr);
+		for (Resize& r : list) {
+			be->release(*r.p);
+			device_bytes -= static_cast<long long>(r.tile_bytes) * arena_tiles;
+			*r.p = r.fresh;
+		}
+		// the table-mode lane arrays are re-created at their next upload
+		const long long lane_array_bytes = static_cast<long long>(arena_tiles) * kLanes * static_cast<long long>(sizeof(int32_t));
+		if (lane_send_dev) {
+			be->release(lane_send_dev);
+			lane_send_dev = nullptr;
+			device_bytes -= lane_array_bytes;
+		}
+		for (int s = 0; s < kMaxSlots; ++s) {
+			if (lane_class_dev[s]) {
+				be->release(lane_class_dev[s]);
+				lane_class_dev[s] = nullptr;
+				device_bytes -= lane_array_bytes;
+			}
+		}
+		arena_tiles = new_tiles;
+		const size_t lanes = static_cast<size_t>(new_tiles) * kLanes;
+		for (int s = 0; s < kMaxSlots; ++s) {
+			fx_class[s].resize(lanes, 0);
+		}
+		send_class.resize(lanes, send_class[0]);
+		pending.resize(lanes, 0);
+		stream_of_lane.resize(lanes, -1);
+		tile_key.resize(static_cast<size_t>(new_tiles));
+		tile_active.resize(static_cast<size_t>(new_tiles), 0);
+		return ok;
+	}
+
+	// The configuration vectors become lane-indexed over the arena; the streams stay where they are until the next mix.
+	void enter_placed()
+	{
+		const size_t lanes = static_cast<size_t>(arena_tiles) * kLanes;
+		lane_of_stream.resize(static_cast<size_t>(streams));
+		stream_of_lane.assign(lanes, -1);
+		for (int s = 0; s < streams; ++s) {
+			lane_of_stream[static_cast<size_t>(s)] = s;
+			stream_of_lane[static_cast<size_t>(s)] = s;
+		}
+		for (int s = 0; s < kMaxSlots; ++s) {
+			fx_class[s].resize(lanes, 0);
+		}
+		send_class.resize(lanes, send_class[0]);
+		pending.resize(lanes, 0);
+		tile_key.assign(static_cast<size_t>(arena_tiles), GroupKey());
+		tile_active.assign(static_cast<size_t>(arena_tiles), 0);
+		refill_padding = true;
+		placed = true;
+	}
+
+	// Every stream back to lane = stream, the configuration vectors back to caller order.
+	bool leave_placed()
+	{
+		std::vector<std::pair<int32_t, int32_t>> moves;
+		for (int s = 0; s < streams; ++s) {
+			if (lane_of_stream[static_cast<size_t>(s)] != s) {
+				moves.push_back(std::make_pair(lane_of_stream[static_cast<size_t>(s)], s));
+			}
+		}
+		if (!move_lanes(moves)) {
+			return false;
+		}
+		auto to_caller = [&](auto& v) {
+			auto out = v;
+			out.resize(static_cast<size_t>(streams));
+			for (int s = 0; s < streams; ++s) {
+				out[static_cast<size_t>(s)] = v[static_cast<size_t>(lane_of_stream[static_cast<size_t>(s)])];
+			}
+			v.swap(out);
+		};
+		for (int s = 0; s < kMaxSlots; ++s) {
+			to_caller(fx_class[s]);
+		}
+		to_caller(send_class);
+		to_caller(pending);
+		placed = false;
+		lane_of_stream.clear();
+		stream_of_lane.clear();
+		tile_key.clear();
+		tile_active.clear();
+		return true;
+	}
+
+	// The placement itself (run before the groups are built, engine quiesced).  Keyed on the full GroupKey -- pending bits
+	// included, so that the block that consumes an update is class-pure as well.  Afterwards:
+	//   1. every tile that holds a caller stream holds one key; its padding lanes carry that key;
+	//   2. a stream already in a pure tile of its key is not moved (except by 3), so changing k streams moves about k;
+	//   3. a key of n streams spans at most ceil(n / 32) + 1 tiles, else it is re-packed into ceil(n / 32);
+	//   4. freed tiles are reused before the arenas grow; they never shrink.
+	bool place_streams()
+	{
+		place_oom = false;
+		const int T = arena_tiles;
+		std::map<GroupKey, int> ids;
+		std::vector<GroupKey> keys;
+		std::vector<int> kid(static_cast<size_t>(streams));
+		for (int s = 0; s < streams; ++s) {
+			const GroupKey k = key_of(lane_of_stream[static_cast<size_t>(s)]);
+			auto it = ids.emplace(k, static_cast<int>(keys.size()));
+			if (it.second) {
+				keys.push_back(k);
+			}
+			kid[static_cast<size_t>(s)] = it.first->second;
+		}
+		const int K = static_cast<int>(keys.size());
+		// each tile stays with the key most of its streams have (ties: the key seen first); the others move
+		std::vector<int> owner(static_cast<size_t>(T), -1), kept(static_cast<size_t>(T), 0);
+		for (int t = 0; t < T; ++t) {
+			int ids_here[kLanes], counts[kLanes], distinct = 0;
+			for (int l = t * kLanes; l < (t + 1) * kLanes; ++l) {
+				const int s = stream_of_lane[static_cast<size_t>(l)];
+				if (s < 0) {
+					continue;
+				}
+				const int k = kid[static_cast<size_t>(s)];
+				int j = 0;
+				while (j < distinct && ids_here[j] != k) {
+					++j;
+				}
+				if (j == distinct) {
+					ids_here[distinct] = k;
+					counts[distinct++] = 0;
+				}
+				++counts[j];
+			}
+			for (int j = 0; j < distinct; ++j) {
+				if (counts[j] > kept[static_cast<size_t>(t)] || (counts[j] == kept[static_cast<size_t>(t)] && ids_here[j] < owner[static_cast<size_t>(t)])) {
+					owner[static_cast<size_t>(t)] = ids_here[j];
+					kept[static_cast<size_t>(t)] = counts[j];
+				}
+			}
+		}
+		std::vector<std::vector<int>> owned(static_cast<size_t>(K)), movers(static_cast<size_t>(K));
+		std::vector<int> members(static_cast<size_t>(K), 0);
+		for (int t = 0; t < T; ++t) {
+			if (owner[static_cast<size_t>(t)] >= 0) {
+				owned[static_cast<size_t>(owner[static_cast<size_t>(t)])].push_back(t);
+			}
+		}
+		for (int s = 0; s < streams; ++s) {
+			const int k = kid[static_cast<size_t>(s)];
+			++members[static_cast<size_t>(k)];
+			if (owner[static_cast<size_t>(lane_of_stream[static_cast<size_t>(s)] / kLanes)] != k) {
+				movers[static_cast<size_t>(k)].push_back(s);
+			}
+		}
+		auto new_tiles_for = [&](int k) {
+			long long kept_k = 0;
+			for (int t : owned[static_cast<size_t>(k)]) {
+				kept_k += kept[static_cast<size_t>(t)];
+			}
+			const long long spare = static_cast<long long>(owned[static_cast<size_t>(k)].size()) * kLanes - kept_k;
+			const long long extra = static_cast<long long>(movers[static_cast<size_t>(k)].size()) - spare;
+			return static_cast<int>(extra > 0 ? (extra + kLanes - 1) / kLanes : 0);
+		};
+		for (int k = 0; k < K; ++k) {
+			std::vector<int>& mine = owned[static_cast<size_t>(k)];
+			const int bound = (members[static_cast<size_t>(k)] + kLanes - 1) / kLanes;
+			if (static_cast<int>(mine.size()) + new_tiles_for(k) <= bound + 1) {
+				continue;
+			}
+			// re-pack: keep the fullest `bound` tiles, the streams of the others move into their free lanes
+			std::stable_sort(mine.begin(), mine.end(), [&](int a, int b) { return kept[static_cast<size_t>(a)] > kept[static_cast<size_t>(b)]; });
+			for (size_t i = static_cast<size_t>(bound); i < mine.size(); ++i) {
+				const int t = mine[i];
+				owner[static_cast<size_t>(t)] = -1;
+				for (int l = t * kLanes; l < (t + 1) * kLanes; ++l) {
+					const int s = stream_of_lane[static_cast<size_t>(l)];
+					if (s >= 0 && kid[static_cast<size_t>(s)] == k) {
+						movers[static_cast<size_t>(k)].push_back(s);
+					}
+				}
+			}
+			mine.resize(std::min(mine.size(), static_cast<size_t>(bound)));
+			std::sort(movers[static_cast<size_t>(k)].begin(), movers[static_cast<size_t>(k)].end());
+		}
+		// new tiles: freed ones first (lowest index), then growth
+		std::vector<int> free_tiles;
+		for (int t = 0; t < T; ++t) {
+			if (owner[static_cast<size_t>(t)] < 0) {
+				free_tiles.push_back(t);
+			}
+		}
+		size_t next_free = 0;
+		int new_T = T;
+		for (int k = 0; k < K; ++k) {
+			for (int n = new_tiles_for(k); n > 0; --n) {
+				owned[static_cast<size_t>(k)].push_back(next_free < free_tiles.size() ? free_tiles[next_free++] : new_T++);
+			}
+		}
+		// Growing copies every arena: grow by an eighth or by one spare tile per key, whichever is more, so that the new
+		// (class, pending) tiles of later updates and the partial tiles they leave behind find free tiles instead of
+		// another copy of the whole arena.
+		if (new_T > T) {
+			new_T = std::max(new_T + K, T + (T + 7) / 8);
+		}
+		if (new_T > T && !grow_arena(new_T)) {
+			place_oom = true;
+			return false;
+		}
+		owner.resize(static_cast<size_t>(new_T), -1);
+		for (int k = 0; k < K; ++k) {
+			for (int t : owned[static_cast<size_t>(k)]) {
+				owner[static_cast<size_t>(t)] = k;
+			}
+		}
+		// movers into the free lanes of their key's tiles, in stream order
+		std::vector<int32_t> next_sol(stream_of_lane);
+		std::vector<uint8_t> touched(static_cast<size_t>(new_T), 0);
+		for (int k = 0; k < K; ++k) {
+			for (int s : movers[static_cast<size_t>(k)]) {
+				const int l = lane_of_stream[static_cast<size_t>(s)];
+				next_sol[static_cast<size_t>(l)] = -1;
+				touched[static_cast<size_t>(l / kLanes)] = 1;
+			}
+		}
+		std::vector<std::pair<int32_t, int32_t>> moves;
+		for (int k = 0; k < K; ++k) {
+			size_t m = 0;
+			for (int t : owned[static_cast<size_t>(k)]) {
+				for (int l = t * kLanes; l < (t + 1) * kLanes && m < movers[static_cast<size_t>(k)].size(); ++l) {
+					if (next_sol[static_cast<size_t>(l)] < 0) {
+						const int s = movers[static_cast<size_t>(k)][m++];
+						next_sol[static_cast<size_t>(l)] = s;
+						touched[static_cast<size_t>(t)] = 1;
+						if (lane_of_stream[static_cast<size_t>(s)] != l) {
+							moves.push_back(std::make_pair(lane_of_stream[static_cast<size_t>(s)], l));
+						}
+					}
+				}
+			}
+		}
+		if (!move_lanes(moves)) {
+			return false;
+		}
+		for (int s = 0; s < kMaxSlots; ++s) {
+			const std::vector<int> before(fx_class[s]);
+			for (const auto& mv : moves) {
+				fx_class[s][static_cast<size_t>(mv.second)] = before[static_cast<size_t>(mv.first)];
+			}
+		}
+		const std::vector<int> send_before(send_class);
+		const std::vector<uint8_t> pending_before(pending);
+		for (const auto& mv : moves) {
+			send_class[static_cast<size_t>(mv.second)] = send_before[static_cast<size_t>(mv.first)];
+			pending[static_cast<size_t>(mv.second)] = pending_before[static_cast<size_t>(mv.first)];
+		}
+		stream_of_lane.swap(next_sol);
+		for (const auto& mv : moves) {
+			lane_of_stream[static_cast<size_t>(stream_of_lane[static_cast<size_t>(mv.second)])] = mv.second;
+		}
+		// padding lanes: their tile's key, and (where the tile changed) a tile-mate's slot and send state -- the kernels'
+		// warp-uniform checks (ring offsets) then see the padding lanes agree with the tile
+		std::vector<int32_t> pad_to, pad_from;
+		for (int t = 0; t < new_T; ++t) {
+			const int k = owner[static_cast<size_t>(t)];
+			int mate = -1;
+			for (int l = t * kLanes; l < (t + 1) * kLanes && mate < 0; ++l) {
+				mate = stream_of_lane[static_cast<size_t>(l)] >= 0 ? l : -1;
+			}
+			const bool active = mate >= 0;
+			const bool changed = refill_padding || touched[static_cast<size_t>(t)] || !tile_active[static_cast<size_t>(t)] ||
+				!(tile_key[static_cast<size_t>(t)] == keys[static_cast<size_t>(std::max(k, 0))]);
+			tile_active[static_cast<size_t>(t)] = active ? 1 : 0;
+			if (!active) {
+				continue;
+			}
+			const GroupKey& key = keys[static_cast<size_t>(k)];
+			tile_key[static_cast<size_t>(t)] = key;
+			for (int l = t * kLanes; l < (t + 1) * kLanes; ++l) {
+				if (stream_of_lane[static_cast<size_t>(l)] >= 0) {
+					continue;
+				}
+				for (int s = 0; s < kMaxSlots; ++s) {
+					fx_class[s][static_cast<size_t>(l)] = key.fx[s];
+				}
+				send_class[static_cast<size_t>(l)] = key.send;
+				pending[static_cast<size_t>(l)] = static_cast<uint8_t>(key.pending);
+				if (changed) {
+					pad_to.push_back(l);
+					pad_from.push_back(mate);
+				}
+			}
+		}
+		refill_padding = false;
+		if (!pad_to.empty()) {
+			std::vector<int32_t> lists(pad_from);
+			lists.insert(lists.end(), pad_to.begin(), pad_to.end());
+			if (!upload_lane_list(lists)) {
+				return false;
+			}
+			const int n = static_cast<int>(pad_to.size());
+			for (const Arena& a : arenas(false)) {
+				const long long ts = static_cast<long long>(a.words) * kLanes;
+				if (!be->copy_lanes(a.base, ts, 0, a.base, ts, 0, a.words, lane_list_dev, lane_list_dev + n, n, nullptr)) {
+					return false;
+				}
+			}
+		}
+		return grow(stream_of_lane_dev, stream_of_lane_cap, stream_of_lane.size()) &&
+			be->upload(stream_of_lane_dev, stream_of_lane.data(), stream_of_lane.size() * sizeof(int32_t), nullptr) && be->sync(nullptr);
+	}
+
+	// Groups of a placed engine: the active tiles only, every one of them whole and of one key.  Each slot signature with
+	// enough keys gets ONE class-per-tile launch; the remaining keys run per key (a handful) or in table mode.  For blocks
+	// the class-per-tile kernels cannot take (frames < 2), fallback_groups covers every key without them.
+	bool build_placed_groups()
+	{
+		constexpr size_t kTableModeMinGroups = 8; // as in rebuild_groups
+		constexpr size_t kMultiMinGroups = 3;     // as in build_multi
+		groups.clear();
+		fallback_groups.clear();
+		multi_kernel = -1;
+		std::map<GroupKey, std::vector<TileRef>> by_key;
+		for (int t = 0; t < arena_tiles; ++t) {
+			if (tile_active[static_cast<size_t>(t)]) {
+				by_key[tile_key[static_cast<size_t>(t)]].push_back(TileRef{static_cast<uint32_t>(t), 0xFFFFFFFFU});
+			}
+		}
+		std::vector<TileRef> all;
+		std::vector<MixClassEntry> table;
+		std::vector<int32_t> tile_class(static_cast<size_t>(arena_tiles), -1);
+		std::map<std::vector<int>, std::vector<const GroupKey*>> by_signature;
+		std::map<GroupKey, std::vector<TileRef>> rest;
+		const bool multi_ok = be->has_relay() && (channels == 1 || channels == 2) && (family == 2 || family == 4);
+		for (const auto& kv : by_key) {
+			int kinds[kMaxSlots];
+			bool ok = multi_ok && multi_kinds_of(kv.first, kinds);
+			int active = 0;
+			for (int s = 0; s < kMaxSlots; ++s) {
+				active += kinds[s] != kKindNull ? 1 : 0;
+			}
+			if (ok && active >= 1) {
+				by_signature[std::vector<int>(kinds, kinds + kMaxSlots)].push_back(&kv.first);
+			} else {
+				rest.insert(kv);
+			}
+		}
+		const KernelInfo* infos = kernel_infos();
+		for (const auto& sig : by_signature) {
+			if (sig.second.size() < kMultiMinGroups) { // one or two big classes: a constant-bank launch each is faster
+				for (const GroupKey* k : sig.second) {
+					rest.emplace(*k, by_key[*k]);
+				}
+				continue;
+			}
+			const int* kinds = sig.first.data();
+			const bool chain = channels == 2 && std::memcmp(infos[kChainStereo].kind, kinds, sizeof(int) * kMaxSlots) == 0;
+			bool heavy = false;
+			for (int s = 0; s < kMaxSlots; ++s) {
+				heavy = heavy || kinds[s] == kKindReverb;
+			}
+			Group g;
+			g.key = *sig.second.front();
+			g.key.pending = 0;
+			g.multi = true;
+			g.tile_begin = all.size();
+			for (const GroupKey* k : sig.second) {
+				for (const TileRef& t : by_key[*k]) {
+					tile_class[t.tile] = static_cast<int32_t>(table.size());
+					all.push_back(t);
+				}
+				table.push_back(multi_entry(*k, kinds, chain));
+				g.key.pending |= k->pending;
+			}
+			g.tile_count = static_cast<int>(all.size() - g.tile_begin);
+			g.multi_kernel = chain ? kMultiChainStereo :
+				channels == 1 ? (heavy ? kRelayMultiMonoHeavy : kRelayMultiMono) : (heavy ? kRelayMultiStereoHeavy : kRelayMultiStereo);
+			std::memcpy(g.multi_kinds, kinds, sizeof(g.multi_kinds));
+			groups.push_back(g);
+		}
+		bool tables_needed = false;
+		auto add_groups = [&](const std::map<GroupKey, std::vector<TileRef>>& keyed, std::vector<Group>& out) {
+			const bool table_mode = keyed.size() > kTableModeMinGroups;
+			std::map<GroupKey, std::vector<TileRef>> by_kinds;
+			const std::map<GroupKey, std::vector<TileRef>>* src = &keyed;
+			if (table_mode) {
+				tables_needed = true;
+				for (const auto& kv : keyed) {
+					GroupKey k = kv.first;
+					for (int i = 0; i < kMaxSlots; ++i) {
+						k.fx[i] = kind_of_type(classes[static_cast<size_t>(k.fx[i])].type);
+					}
+					k.send = 0;
+					std::vector<TileRef>& v = by_kinds[k];
+					v.insert(v.end(), kv.second.begin(), kv.second.end());
+				}
+				src = &by_kinds;
+			}
+			for (const auto& kv : *src) {
+				Group g;
+				g.key = kv.first;
+				g.table = table_mode;
+				g.full_tiles = true;
+				g.tile_begin = all.size();
+				g.tile_count = static_cast<int>(kv.second.size());
+				all.insert(all.end(), kv.second.begin(), kv.second.end());
+				out.push_back(g);
+			}
+		};
+		add_groups(rest, groups);
+		if (!table.empty()) {
+			add_groups(by_key, fallback_groups);
+		}
+		if (tables_needed && !upload_tables()) {
+			return false;
+		}
+		if (all.size() > tile_list_cap) {
+			be->sync(nullptr);
+			be->release(tile_list);
+			device_bytes -= static_cast<long long>(tile_list_cap * sizeof(TileRef));
+			tile_list_cap = all.size() * 2;
+			tile_list = static_cast<TileRef*>(dev_alloc(tile_list_cap * sizeof(TileRef)));
+			if (!tile_list) {
+				tile_list_cap = 0;
+				return false;
+			}
+		}
+		if (!all.empty() && !be->upload(tile_list, all.data(), all.size() * sizeof(TileRef), nullptr)) {
+			return false;
+		}
+		if (!table.empty()) {
+			if (!grow(class_table_dev, class_table_cap, table.size())) {
+				return false;
+			}
+			if (!tile_class_dev && !(tile_class_dev = static_cast<int32_t*>(dev_alloc(static_cast<size_t>(arena_tiles) * sizeof(int32_t))))) {
+				return false;
+			}
+			if (!be->upload(class_table_dev, table.data(), table.size() * sizeof(MixClassEntry), nullptr) ||
+				!be->upload(tile_class_dev, tile_class.data(), tile_class.size() * sizeof(int32_t), nullptr)) {
+				return false;
+			}
+		}
+		if (!be->sync(nullptr)) {
+			return false;
+		}
+		groups_dirty = false;
+		return true;
+	}
+
+	// Snapshot / restore of a placed engine: every arena in caller stream order (stream s at tile s / 32, lane s % 32;
+	// zeros past the last stream), `tiles` tiles per arena, gathered through the scratch arena in chunks of whole tiles.
+	// (snapshot: `out` receives the arenas; restore: `in` holds them)
+	bool canonical_state(char* out, const char* in)
+	{
+		std::vector<int32_t> canon(static_cast<size_t>(tiles) * kLanes, -1);
+		for (int s = 0; s < streams; ++s) {
+			canon[static_cast<size_t>(s)] = lane_of_stream[static_cast<size_t>(s)];
+		}
+		if (!upload_lane_list(canon)) {
+			return false;
+		}
+		bool ok = true;
+		for (const Arena& a : arenas(true)) {
+			const size_t tile_words = static_cast<size_t>(a.words) * kLanes;
+			const int per = static_cast<int>(std::max<size_t>(1, std::min<size_t>(static_cast<size_t>(tiles), kMoveScratchWords / tile_words)));
+			ok = ok && ensure_scratch(tile_words * static_cast<size_t>(per));
+			const long long ts = static_cast<long long>(tile_words);
+			for (int t0 = 0; t0 < tiles && ok; t0 += per) {
+				const int nt = std::min(per, tiles - t0);
+				const size_t bytes = tile_words * static_cast<size_t>(nt) * sizeof(uint32_t);
+				const int32_t* lanes = lane_list_dev + static_cast<size_t>(t0) * kLanes;
+				if (in) {
+					ok = be->upload(move_scratch, in, bytes, nullptr) &&
+						be->copy_lanes(a.base, ts, 0, move_scratch, ts, 0, a.words, nullptr, lanes, nt * kLanes, nullptr) && be->sync(nullptr);
+				} else {
+					ok = be->copy_lanes(move_scratch, ts, 0, a.base, ts, 0, a.words, lanes, nullptr, nt * kLanes, nullptr) &&
+						be->download(out, move_scratch, bytes, nullptr) && be->sync(nullptr);
+				}
+				if (in) {
+					in += bytes;
+				} else {
+					out += bytes;
+				}
+			}
+		}
+		return ok;
+	}
+
+	// Class-per-tile eligibility of one key: its slot kinds, and false when it needs the exact kernels (an active send
+	// filter, an unstable filter design).
+	bool multi_kinds_of(const GroupKey& key, int kinds[kMaxSlots]) const
+	{
+		const SendClass& sc = send_classes[static_cast<size_t>(key.send)];
+		bool ok = sc.direct_coef.filter_type == 0;
+		for (int s = 0; s < kMaxSlots; ++s) {
+			const FxClass& fc = classes[static_cast<size_t>(key.fx[s])];
+			kinds[s] = kind_of_type(fc.type);
+			ok = ok && (kinds[s] == kKindNull || sc.aux_coef[s].filter_type == 0) && !(fc.coef.flags & kCoefUnstable);
+		}
+		return ok;
+	}
+
+	// The class-table entry of one key: its coefficient blocks as the kernel arguments would hold them.
+	MixClassEntry multi_entry(const GroupKey& key, const int kinds[kMaxSlots], bool chain) const
+	{
+		Group g;
+		g.key = key;
+		MixArgs a;
+		fill_common(a, g, 2, nullptr, nullptr, OALSFX_LAYOUT_STREAM_MAJOR, 2, 0);
+		MixClassEntry e;
+		std::memset(&e, 0, sizeof(e));
+		int pos = 0;
+		for (int s = 0; s < kMaxSlots; ++s) { // the chain kernel addresses slots by index, the relay by compacted position
+			if (chain || kinds[s] != kKindNull) {
+				fill_slot(a, g, pos, s, false);
+				e.pending |= ((key.pending >> s) & 1U) << pos;
+				++pos;
+			}
+		}
+		sanitize_gains(a);
+		std::memcpy(e.coefs, reinterpret_cast<const char*>(&a) + kMixCoefOffset, kMixCoefBytes);
+		return e;
 	}
 
 	// ---- launching ----------------------------------------------------------------------------------
@@ -736,7 +1385,7 @@ struct oalsfx_engine {
 		std::memset(&a, 0, sizeof(a));
 		a.frames = frames;
 		a.channels = channels;
-		a.num_streams = streams;
+		a.num_streams = lane_count();
 		if (layout == OALSFX_LAYOUT_TILED) {
 			a.io_ts = frames_total * channels * kLanes;
 			a.io_ls = 1;
@@ -823,15 +1472,15 @@ struct oalsfx_engine {
 			MixArgs a;
 			fill_common(a, g, frames, src, dst, layout, frames_total, frame0);
 			a.with_dry = 1;
-			const bool chain = multi_kernel == kMultiChainStereo;
+			const bool chain = g.multi_kernel == kMultiChainStereo;
 			int pos = 0, floats = 0;
 			for (int s = 0; s < kMaxSlots; ++s) {
-				if (chain || multi_kinds[s] != kKindNull) {
+				if (chain || g.multi_kinds[s] != kKindNull) {
 					fill_slot(a, g, pos, s, false); // pointers and strides; the coefficient blocks come from the class table
-					a.relay_kind[pos] = multi_kinds[s];
+					a.relay_kind[pos] = g.multi_kinds[s];
 					a.relay_win[pos] = floats;
-					floats += multi_kinds[s] == kKindReverb ? kPfWarpFloats :
-						(multi_kinds[s] == kKindModDelay || multi_kinds[s] == kKindEcho) ? kFwWarpFloats : 0;
+					floats += g.multi_kinds[s] == kKindReverb ? kPfWarpFloats :
+						(g.multi_kinds[s] == kKindModDelay || g.multi_kinds[s] == kKindEcho) ? kFwWarpFloats : 0;
 					++pos;
 				}
 			}
@@ -841,7 +1490,7 @@ struct oalsfx_engine {
 			a.class_table = class_table_dev;
 			a.tile_class = tile_class_dev;
 			++launches;
-			return mix_launch(multi_kernel, a, stream);
+			return mix_launch(g.multi_kernel, a, stream);
 		}
 		if (g.table) {
 			// key.fx[] holds the kinds; one exact single-effect pass per slot, coefficients from the tables
@@ -1085,6 +1734,7 @@ int oalsfx_engine_create(const oalsfx_engine_desc* desc, oalsfx_engine** out)
 	e->dev = dev;
 	e->streams = desc->num_streams;
 	e->tiles = (desc->num_streams + kLanes - 1) / kLanes;
+	e->arena_tiles = e->tiles;
 	e->channels = dev.channels;
 	e->slots = desc->effect_count;
 	if (const char* fam = std::getenv("OALSFX_KERNEL")) {
@@ -1172,18 +1822,20 @@ int oalsfx_engine_set_effect(oalsfx_engine* e, int first_stream, int n_streams, 
 	}
 	// A type change constructs a fresh effect state (oalsfxpp.cpp:2692-2698): zero the slot state and
 	// the rings of exactly those streams.
-	std::vector<TileRef> reset;
+	// (the streams' lanes: placed streams sit in any order, so the tiles are collected by index)
+	std::map<uint32_t, uint32_t> reset_masks;
 	for (int s = first_stream; s < first_stream + n_streams; ++s) {
-		int& cur = e->fx_class[slot][static_cast<size_t>(s)];
+		const int lane = e->lane_of(s);
+		int& cur = e->fx_class[slot][static_cast<size_t>(lane)];
 		if (e->classes[static_cast<size_t>(cur)].type != effect_type) {
-			const uint32_t tile = static_cast<uint32_t>(s / kLanes);
-			if (reset.empty() || reset.back().tile != tile) {
-				reset.push_back(TileRef{tile, 0});
-			}
-			reset.back().mask |= 1U << (s % kLanes);
+			reset_masks[static_cast<uint32_t>(lane / kLanes)] |= 1U << (lane % kLanes);
 		}
 		cur = id;
-		e->pending[static_cast<size_t>(s)] |= static_cast<uint8_t>(1U << slot); // is_props_changed_ (oalsfxpp.cpp:2707)
+		e->pending[static_cast<size_t>(lane)] |= static_cast<uint8_t>(1U << slot); // is_props_changed_ (oalsfxpp.cpp:2707)
+	}
+	std::vector<TileRef> reset;
+	for (const auto& tm : reset_masks) {
+		reset.push_back(TileRef{tm.first, tm.second});
 	}
 	if (!reset.empty()) {
 		const int n = static_cast<int>(reset.size());
@@ -1217,7 +1869,7 @@ int oalsfx_engine_set_sends(oalsfx_engine* e, int first_stream, int n_streams, c
 	}
 	const int id = e->send_class_for(d, a);
 	for (int s = first_stream; s < first_stream + n_streams; ++s) {
-		e->send_class[static_cast<size_t>(s)] = id;
+		e->send_class[static_cast<size_t>(e->lane_of(s))] = id;
 	}
 	e->groups_dirty = true;
 	return OALSFX_OK;
@@ -1329,20 +1981,62 @@ int oalsfx_engine_mix(oalsfx_engine* e, int frames, const float* src, float* dst
 		return e->fail(OALSFX_ERR_ARGUMENT, "Unknown pointer space.");
 	}
 
+	// caller strides of the buffers (a placed engine permutes each block into lane order and back)
+	const long long io_ts = static_cast<long long>(frames) * e->channels * kLanes;
+	const long long io_ls = layout == OALSFX_LAYOUT_TILED ? 1 : static_cast<long long>(frames) * e->channels;
+	const long long io_fs = layout == OALSFX_LAYOUT_TILED ? static_cast<long long>(e->channels) * kLanes : e->channels;
+	const long long io_cs = layout == OALSFX_LAYOUT_TILED ? kLanes : 1;
 	bool first_block = true;
 	for (int done = 0; done < frames;) {
 		const int todo = std::min(frames - done, kMaxBlockFrames); // oalsfxpp.cpp:3818-3826
 		if (e->groups_dirty && !e->rebuild_groups()) {
+			if (e->place_oom) {
+				return e->fail(OALSFX_ERR_MEMORY, "Placement could not grow the arenas: " + e->be->error());
+			}
 			return e->fail(OALSFX_ERR_DEVICE, "Group table upload failed: " + e->be->error());
 		}
+		const float* bsrc = dsrc;
+		float* bdst = ddst;
+		int blayout = layout;
+		long long btotal = frames, bframe0 = done;
+		if (e->placed) {
+			const size_t need = static_cast<size_t>(e->arena_tiles) * kLanes * static_cast<size_t>(std::min(frames, kMaxBlockFrames)) *
+				static_cast<size_t>(e->channels);
+			if (need > e->io_cap) {
+				e->be->sync(cuda_stream);
+				e->be->release(e->io_in);
+				e->be->release(e->io_out);
+				e->device_bytes -= static_cast<long long>(e->io_cap) * 2 * sizeof(float);
+				e->io_in = static_cast<float*>(e->dev_alloc(need * sizeof(float)));
+				e->io_out = static_cast<float*>(e->dev_alloc(need * sizeof(float)));
+				e->io_cap = need;
+				if (!e->io_in || !e->io_out) {
+					e->io_cap = 0;
+					return e->fail(OALSFX_ERR_MEMORY, "Placement block allocation failed: " + e->be->error());
+				}
+			}
+			if (!e->be->gather_io(dsrc + done * io_fs, io_ts, io_ls, io_fs, io_cs, e->stream_of_lane_dev, e->arena_tiles, todo,
+					e->channels, e->io_in, cuda_stream)) {
+				return e->fail(OALSFX_ERR_DEVICE, e->be->error());
+			}
+			bsrc = e->io_in;
+			bdst = e->io_out;
+			blayout = OALSFX_LAYOUT_TILED;
+			btotal = todo;
+			bframe0 = 0;
+		}
 		bool had_pending = false;
-		const bool use_fallback = e->groups.size() == 1 && e->groups[0].multi && todo < 2;
+		const bool use_fallback = !e->fallback_groups.empty() && todo < 2; // (only class-per-tile launches have fallback groups)
 		had_pending = use_fallback && e->groups[0].key.pending != 0;
 		for (const Group& g : (use_fallback ? e->fallback_groups : e->groups)) {
 			had_pending = had_pending || g.key.pending != 0;
-			if (!e->launch_group(g, todo, dsrc, ddst, layout, frames, done, first_block, cuda_stream)) {
+			if (!e->launch_group(g, todo, bsrc, bdst, blayout, btotal, bframe0, first_block, cuda_stream)) {
 				return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 			}
+		}
+		if (e->placed && !e->be->scatter_io(e->io_out, e->stream_of_lane_dev, e->arena_tiles, todo, e->channels, ddst + done * io_fs,
+				io_ts, io_ls, io_fs, io_cs, cuda_stream)) {
+			return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 		}
 		if (had_pending) {
 			std::fill(e->pending.begin(), e->pending.end(), static_cast<uint8_t>(0));
@@ -1529,6 +2223,13 @@ int oalsfx_engine_snapshot(oalsfx_engine* e, void* dst, size_t bytes)
 	char* out = static_cast<char*>(dst);
 	std::memcpy(out, &h, sizeof(h));
 	out += sizeof(h);
+	if (e->placed) {
+		for (int s = 0; s < e->streams; ++s) {
+			out[s] = static_cast<char>(e->pending[static_cast<size_t>(e->lane_of(s))]);
+		}
+		out += e->streams;
+		return e->canonical_state(out, nullptr) ? OALSFX_OK : e->fail(OALSFX_ERR_DEVICE, e->be->error());
+	}
 	std::memcpy(out, e->pending.data(), static_cast<size_t>(e->streams));
 	out += e->streams;
 	bool ok = true;
@@ -1565,10 +2266,18 @@ int oalsfx_engine_restore(oalsfx_engine* e, const void* src, size_t bytes)
 		return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 	}
 	const char* in = static_cast<const char*>(src) + sizeof(SnapshotHeader);
-	std::memcpy(e->pending.data(), in, static_cast<size_t>(e->streams));
-	in += e->streams;
 	e->groups_dirty = true;
 	e->frames_since_update = 128; // unknown history: let the steady-state kernels try (they check the stream state)
+	if (e->placed) {
+		for (int s = 0; s < e->streams; ++s) {
+			e->pending[static_cast<size_t>(e->lane_of(s))] = static_cast<uint8_t>(in[s]);
+		}
+		in += e->streams;
+		e->refill_padding = true;
+		return e->canonical_state(nullptr, in) ? OALSFX_OK : e->fail(OALSFX_ERR_DEVICE, e->be->error());
+	}
+	std::memcpy(e->pending.data(), in, static_cast<size_t>(e->streams));
+	in += e->streams;
 	bool ok = true;
 	for (int s = 0; s < e->slots && ok; ++s) {
 		const size_t ring_bytes = static_cast<size_t>(e->tiles) * static_cast<size_t>(e->ring_cap[s]) * kLanes * sizeof(float);
@@ -1590,16 +2299,16 @@ int oalsfx_engine_debug_state(oalsfx_engine* e, int stream, int slot, int32_t ou
 	if (!e || !out || stream < 0 || stream >= e->streams || slot < 0 || slot >= e->slots) {
 		return e ? e->fail(OALSFX_ERR_ARGUMENT, "Bad debug_state arguments.") : OALSFX_ERR_ARGUMENT;
 	}
+	const int lane = e->lane_of(stream);
 	std::vector<uint32_t> words(static_cast<size_t>(kSlotStateWords) * kLanes);
-	const uint32_t* p = e->slot_state[slot] + static_cast<size_t>(stream / kLanes) * kSlotStateWords * kLanes;
+	const uint32_t* p = e->slot_state[slot] + static_cast<size_t>(lane / kLanes) * kSlotStateWords * kLanes;
 	if (!e->quiesce() || !e->be->download(words.data(), p, words.size() * sizeof(uint32_t), nullptr) ||
 		!e->be->sync(nullptr)) {
 		return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 	}
-	const int lane = stream % kLanes;
-	auto word = [&](size_t i) { return static_cast<int32_t>(words[i * kLanes + static_cast<size_t>(lane)]); };
+	auto word = [&](size_t i) { return static_cast<int32_t>(words[i * kLanes + static_cast<size_t>(lane % kLanes)]); };
 	out[0] = out[1] = out[2] = out[3] = 0;
-	const int type = e->classes[static_cast<size_t>(e->fx_class[slot][static_cast<size_t>(stream)])].type;
+	const int type = e->classes[static_cast<size_t>(e->fx_class[slot][static_cast<size_t>(lane)])].type;
 	switch (kind_of_type(type)) {
 	case kKindModDelay: out[0] = word(offsetof(FxModDelay::State, offset) / 4); break;
 	case kKindEcho: out[0] = word(offsetof(FxEcho::State, offset) / 4); break;
@@ -1612,6 +2321,41 @@ int oalsfx_engine_debug_state(oalsfx_engine* e, int stream, int slot, int32_t ou
 	default: break;
 	}
 	return OALSFX_OK;
+}
+
+int oalsfx_engine_set_placement(oalsfx_engine* e, int mode)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	if (mode != OALSFX_PLACEMENT_CALLER && mode != OALSFX_PLACEMENT_AUTO) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "Unknown placement mode.");
+	}
+	if (!e->quiesce()) {
+		return e->fail(OALSFX_ERR_DEVICE, e->be->error());
+	}
+	e->placement = mode;
+	if (mode == OALSFX_PLACEMENT_AUTO && !e->placed) {
+		e->enter_placed();
+	} else if (mode == OALSFX_PLACEMENT_CALLER && e->placed && !e->leave_placed()) {
+		return e->fail(OALSFX_ERR_DEVICE, "Moving the streams back failed: " + e->be->error());
+	}
+	e->groups_dirty = true;
+	return OALSFX_OK;
+}
+
+long long oalsfx_engine_lanes(oalsfx_engine* e, int32_t* lane_of_stream, int n)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	if (n < 0 || n > e->streams || (n > 0 && !lane_of_stream)) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "Bad lanes arguments.");
+	}
+	for (int s = 0; s < n; ++s) {
+		lane_of_stream[s] = e->lane_of(s);
+	}
+	return static_cast<long long>(e->placed ? e->arena_tiles : e->tiles) * kLanes;
 }
 
 long long oalsfx_engine_launch_count(const oalsfx_engine* e) { return e ? e->launches : 0; }

@@ -95,6 +95,10 @@ def bind(lib):
     lib.oalsfx_engine_snapshot.restype = i32
     lib.oalsfx_engine_restore.argtypes = [vp, vp, C.c_size_t]
     lib.oalsfx_engine_restore.restype = i32
+    lib.oalsfx_engine_set_placement.argtypes = [vp, i32]
+    lib.oalsfx_engine_set_placement.restype = i32
+    lib.oalsfx_engine_lanes.argtypes = [vp, vp, i32]
+    lib.oalsfx_engine_lanes.restype = C.c_longlong
     return lib
 
 
@@ -106,6 +110,7 @@ EXPORTED_SYMBOLS = (
     "oalsfx_last_error", "oalsfx_build_info", "oalsfx_effect_defaults", "oalsfx_effect_normalize",
     "oalsfx_reverb_preset", "oalsfx_reverb_preset_name", "oalsfx_pcm_to_float", "oalsfx_float_to_s16",
     "oalsfx_engine_snapshot_size", "oalsfx_engine_snapshot", "oalsfx_engine_restore",
+    "oalsfx_engine_set_placement", "oalsfx_engine_lanes",
 )
 
 _LIB = None
@@ -284,6 +289,28 @@ class Engine:
     def restore(self, snapshot):
         snapshot = np.ascontiguousarray(snapshot, dtype=np.uint8)
         self._check(self.lib.oalsfx_engine_restore(self._h, snapshot.ctypes.data, snapshot.size))
+
+    _PLACEMENT = {"caller": 0, "auto": 1}
+
+    def set_placement(self, mode):
+        """"caller" (default: engine lane of stream s is s) or "auto": the engine moves streams between its lanes so
+        that every 32-stream tile holds one parameter class.  Stream indices and buffers keep the caller's order."""
+        if mode not in self._PLACEMENT:
+            raise ValueError(f"placement must be one of {sorted(self._PLACEMENT)}")
+        self._check(self.lib.oalsfx_engine_set_placement(self._h, self._PLACEMENT[mode]))
+
+    @property
+    def lane_of_stream(self):
+        """The engine lane that holds each caller stream now (int32 array of num_streams)."""
+        return self.lanes()[0]
+
+    def lanes(self):
+        """(lane_of_stream, the engine's lane count: a multiple of 32)."""
+        out = np.empty(self.num_streams, dtype=np.int32)
+        n = self.lib.oalsfx_engine_lanes(self._h, out.ctypes.data, self.num_streams)
+        if n < 0:
+            self._check(int(n))
+        return out, int(n)
 
     @property
     def launch_count(self):
