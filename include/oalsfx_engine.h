@@ -71,10 +71,32 @@ int oalsfx_engine_set_effect(oalsfx_engine* e, int first_stream, int n_streams, 
 int oalsfx_engine_set_sends(oalsfx_engine* e, int first_stream, int n_streams,
 	const float* direct, const float* aux);
 
+/* Voice lifecycle.  In the reference each voice is one Api, and a host mixes only the voices that play; a voice it does
+ * not mix keeps its delay lines and filter histories as they are.
+ * oalsfx_engine_set_active: streams [first_stream, first_stream + n_streams) are mixed (active != 0, the default for
+ * every stream) or paused.  From the next mix on the engine does not process a paused stream -- it is an Api whose mix is
+ * not called: its rings, slot state, send filter histories, ring offsets, LFO / modulator phases, tap cross-fade counter
+ * and pending updates stay exactly as they are, and it costs no mix work.  Its src rows are not read and its dst rows
+ * receive +0.0f in every frame and channel (both layouts, both spaces, mix and mix_bus; so the bus of a block is the sum
+ * over the streams that were mixed).  A resumed stream continues bit for bit like that Api on its next mix.  set_effect /
+ * set_sends on a paused stream behave as always: a type change resets the slot at once, property changes are consumed by
+ * the first block that mixes the stream again.  Activity is configuration, like effect types: snapshots do not hold it
+ * and restore leaves it alone.  Pausing whole 32-stream tiles keeps the fused kernels of the rest; scattered pauses leave
+ * partly paused tiles, which an unplaced engine runs on the slower per-stream path -- OALSFX_PLACEMENT_AUTO packs paused
+ * streams into tiles of their own instead (a pause or resume then costs a lane move, like a preset change).
+ * oalsfx_engine_reset_streams: the streams restart from silence -- every slot's delay lines and state and the send
+ * filter histories are zeroed and every slot holding an effect gets its update again, as from the set_effect that
+ * configured it -- so that each continues like a freshly created engine given the same set_effect / set_sends calls
+ * (a fresh Api with the same effects and sends after apply_changes).  The configuration and the activity flag are kept.
+ * Both wait for the stream the caller last passed in, as set_effect does, and return OALSFX_ERR_ARGUMENT for a bad
+ * range. */
+int oalsfx_engine_set_active(oalsfx_engine* e, int first_stream, int n_streams, int active);
+int oalsfx_engine_reset_streams(oalsfx_engine* e, int first_stream, int n_streams);
+
 /* Ordering: with device buffers oalsfx_engine_mix / mix_bus / reduce_bus / the PCM conversions are ENQUEUED on
  * `cuda_stream` and return at once; consecutive calls on the same stream run in order.  Every other call that touches
- * engine state on the device -- set_effect / set_sends (state reset, arena growth, table uploads at the next mix),
- * snapshot, restore, debug_state, destroy -- first waits for the stream the caller last passed in, so it is safe to
+ * engine state on the device -- set_effect / set_sends / set_active / reset_streams (state reset, arena growth, table
+ * uploads at the next mix), snapshot, restore, debug_state, destroy -- first waits for the stream the caller last passed in, so it is safe to
  * call them at any time, also with cudaStreamNonBlocking streams.  Using several streams on one engine concurrently
  * is the caller's to order.  Precondition of the fused kernels: finite input samples (an Inf / NaN sample times a
  * gain the reference skips as inaudible would reach output channels the reference leaves untouched). */

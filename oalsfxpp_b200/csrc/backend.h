@@ -45,8 +45,10 @@ public:
 	// [src_w0, +words); from[i] < 0 writes zeros, to[i] < 0 skips the entry, a null list is the identity (lane i).
 	// gather_io: dst (TILED, `frames` frames, lane_tiles tiles) lane l = caller stream stream_of_lane[l] of src
 	// (src[(s/32)*ts + (s%32)*ls + f*fs + c*cs]), zeros where stream_of_lane[l] < 0.  scatter_io: the reverse, caller
-	// rows only.  These defaults are place.cuh's host loops over the kernels' element bodies and need device memory the
-	// host can address: the CPU test backend's.  cuda_backend.cu overrides all three with the sm_100a kernels.
+	// rows only, and zeros in the caller row -2 - stream_of_lane[l] of a parked lane (a paused stream).  zero_rows: zeros in
+	// frames [0, frames) of the caller rows rows[0..n) (DEVICE array, ascending).  These defaults are place.cuh's host
+	// loops over the kernels' element bodies and need device memory the host can address: the CPU test backend's.
+	// cuda_backend.cu overrides all four with the sm_100a kernels.
 	virtual bool copy_lanes(uint32_t* dst, long long dst_ts, int dst_w0, const uint32_t* src, long long src_ts, int src_w0,
 		int words, const int32_t* from, const int32_t* to, int n, void*)
 	{
@@ -63,6 +65,12 @@ public:
 		long long ts, long long ls, long long fs, long long cs, void*)
 	{
 		place::scatter_io_host(src, stream_of_lane, lane_tiles, frames, channels, dst, ts, ls, fs, cs);
+		return true;
+	}
+	virtual bool zero_rows(float* dst, long long ts, long long ls, long long fs, long long cs, const int32_t* rows, int n, int frames,
+		int channels, void*)
+	{
+		place::zero_rows_host(dst, ts, ls, fs, cs, rows, n, frames, channels);
 		return true;
 	}
 	virtual bool launch_mix(int kernel_id, const MixArgs& args, void* stream) = 0;

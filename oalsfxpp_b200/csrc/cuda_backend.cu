@@ -402,6 +402,14 @@ public:
 			static_cast<cudaStream_t>(stream)) && check(cudaGetLastError(), "scatter_io_kernel");
 	}
 
+	bool zero_rows(float* dst, long long ts, long long ls, long long fs, long long cs, const int32_t* rows, int n, int frames,
+		int channels, void* stream) override
+	{
+		DeviceScope scope(this);
+		return scope.ok && launch_zero_rows(dst, ts, ls, fs, cs, rows, n, frames, channels, static_cast<cudaStream_t>(stream)) &&
+			check(cudaGetLastError(), "zero_rows_kernel");
+	}
+
 	bool launch_mix(int kernel_id, const MixArgs& args, void* stream) override
 	{
 		DeviceScope scope(this);

@@ -53,6 +53,7 @@ struct GroupKey {
 	int fx[kMaxSlots];
 	int send;
 	uint32_t pending;
+	uint32_t paused;   // 1: the streams are not mixed (oalsfx_engine_set_active).  Last, so that keys of active streams keep their order.
 	bool operator<(const GroupKey& o) const
 	{
 		return std::memcmp(this, &o, sizeof(GroupKey)) < 0;
@@ -84,6 +85,7 @@ struct oalsfx_engine {
 	std::vector<int> fx_class[kMaxSlots];
 	std::vector<int> send_class;
 	std::vector<uint8_t> pending;       // bit s: slot s has an un-consumed `update`
+	std::vector<uint8_t> active;        // 0: paused, the mix neither runs nor reads the stream and writes zeros to its rows
 	// Frames mixed since a launch last carried an update (or the engine was created / restored): a hint for the
 	// kernels that only run streams in the steady state (span.cuh) -- a reverb's tap cross-fade takes 128 frames
 	// from its update on.  The device checks the real per-stream state; this only avoids launches that would fall back.
@@ -147,8 +149,14 @@ struct oalsfx_engine {
 	std::vector<GroupKey> tile_key;     // per arena tile: the key its caller streams share
 	std::vector<uint8_t> tile_active;   // per arena tile: holds a caller stream
 	bool refill_padding = true;         // every padding lane gets its tile-mate's state at the next placement
+	// Device lane map of the I/O passes: stream_of_lane, except that a lane of a paused stream s holds -2 - s (parked:
+	// neither gathered nor mixed; the scatter writes zeros to its caller row).
 	int32_t* stream_of_lane_dev = nullptr;
 	size_t stream_of_lane_cap = 0;
+	// Unplaced engine with paused streams: their caller rows, zeroed after every block's mix launches (zero_rows).
+	int32_t* paused_rows_dev = nullptr;
+	size_t paused_rows_cap = 0;
+	int paused_rows = 0;
 	int32_t* lane_list_dev = nullptr;   // lane lists of copy_lanes
 	size_t lane_list_cap = 0;
 	uint32_t* move_scratch = nullptr;   // bounded staging arena of the lane moves and of snapshot / restore
@@ -256,6 +264,7 @@ struct oalsfx_engine {
 		be->release(stage_in);
 		be->release(stage_out);
 		be->release(stream_of_lane_dev);
+		be->release(paused_rows_dev);
 		be->release(lane_list_dev);
 		be->release(move_scratch);
 		be->release(io_in);
@@ -508,7 +517,19 @@ struct oalsfx_engine {
 		}
 		k.send = send_class[static_cast<size_t>(s)];
 		k.pending = pending[static_cast<size_t>(s)];
+		k.paused = active[static_cast<size_t>(s)] ? 0U : 1U;
 		return k;
+	}
+
+	// After a block that consumed updates: the lanes that were mixed have none left; paused lanes keep theirs for the
+	// block that mixes them again (the reference applies changes at an Api's next mix).
+	void clear_mixed_pending()
+	{
+		for (size_t l = 0; l < pending.size(); ++l) {
+			if (active[l]) {
+				pending[l] = 0;
+			}
+		}
 	}
 
 	template <class T>
@@ -582,23 +603,40 @@ struct oalsfx_engine {
 			return place_streams() && build_placed_groups();
 		}
 		groups.clear();
+		// paused streams: in no tile list, their rows zeroed by one pass per block
+		std::vector<int32_t> paused_list;
+		for (int s = 0; s < streams; ++s) {
+			if (!active[static_cast<size_t>(s)]) {
+				paused_list.push_back(s);
+			}
+		}
+		paused_rows = static_cast<int>(paused_list.size());
+		if (paused_rows > 0 && (!grow(paused_rows_dev, paused_rows_cap, paused_list.size()) ||
+				!be->upload(paused_rows_dev, paused_list.data(), paused_list.size() * sizeof(int32_t), nullptr) || !be->sync(nullptr))) {
+			return false;
+		}
 		const GroupKey k0 = key_of(0);
 		bool uniform = true;
 		for (int s = 1; s < streams && uniform; ++s) {
 			uniform = key_of(s) == k0;
 		}
 		if (uniform) {
-			Group g;
-			g.key = k0;
-			g.identity = true;
-			g.tile_count = tiles;
-			groups.push_back(g);
+			if (!k0.paused) {
+				Group g;
+				g.key = k0;
+				g.identity = true;
+				g.tile_count = tiles;
+				groups.push_back(g);
+			}
 			fallback_groups.clear();
 			groups_dirty = false;
 			return true;
 		}
 		std::map<GroupKey, std::vector<TileRef>> by_key;
 		for (int s = 0; s < streams; ++s) {
+			if (!active[static_cast<size_t>(s)]) {
+				continue;
+			}
 			std::vector<TileRef>& v = by_key[key_of(s)];
 			const uint32_t tile = static_cast<uint32_t>(s / kLanes);
 			if (v.empty() || v.back().tile != tile) {
@@ -616,6 +654,9 @@ struct oalsfx_engine {
 		if (table_mode) {
 			by_key.clear();
 			for (int s = 0; s < streams; ++s) {
+				if (!active[static_cast<size_t>(s)]) {
+					continue;
+				}
 				GroupKey k = key_of(s);
 				for (int i = 0; i < kMaxSlots; ++i) {
 					k.fx[i] = kind_of_type(classes[static_cast<size_t>(k.fx[i])].type);
@@ -657,7 +698,7 @@ struct oalsfx_engine {
 				return false;
 			}
 		}
-		if (!be->upload(tile_list, all.data(), all.size() * sizeof(TileRef), nullptr) || !be->sync(nullptr)) {
+		if ((!all.empty() && !be->upload(tile_list, all.data(), all.size() * sizeof(TileRef), nullptr)) || !be->sync(nullptr)) {
 			return false;
 		}
 		if (!build_multi(full_keys)) {
@@ -736,6 +777,15 @@ struct oalsfx_engine {
 		g.identity = true;
 		g.multi = true;
 		g.tile_count = tiles;
+		if (paused_rows > 0) {
+			// tiles of paused streams are not launched: the tile list of the per-key groups names every other tile once
+			g.identity = false;
+			g.tile_begin = 0;
+			g.tile_count = 0;
+			for (const Group& f : fallback_groups) {
+				g.tile_count += f.tile_count;
+			}
+		}
 		g.multi_kernel = multi_kernel;
 		std::memcpy(g.multi_kinds, multi_kinds, sizeof(multi_kinds));
 		groups.assign(1, g);
@@ -886,6 +936,7 @@ struct oalsfx_engine {
 		}
 		send_class.resize(lanes, send_class[0]);
 		pending.resize(lanes, 0);
+		active.resize(lanes, 1);
 		stream_of_lane.resize(lanes, -1);
 		tile_key.resize(static_cast<size_t>(new_tiles));
 		tile_active.resize(static_cast<size_t>(new_tiles), 0);
@@ -907,6 +958,8 @@ struct oalsfx_engine {
 		}
 		send_class.resize(lanes, send_class[0]);
 		pending.resize(lanes, 0);
+		active.resize(lanes, 1);
+		paused_rows = 0;
 		tile_key.assign(static_cast<size_t>(arena_tiles), GroupKey());
 		tile_active.assign(static_cast<size_t>(arena_tiles), 0);
 		refill_padding = true;
@@ -938,6 +991,7 @@ struct oalsfx_engine {
 		}
 		to_caller(send_class);
 		to_caller(pending);
+		to_caller(active);
 		placed = false;
 		lane_of_stream.clear();
 		stream_of_lane.clear();
@@ -1106,9 +1160,11 @@ struct oalsfx_engine {
 		}
 		const std::vector<int> send_before(send_class);
 		const std::vector<uint8_t> pending_before(pending);
+		const std::vector<uint8_t> active_before(active);
 		for (const auto& mv : moves) {
 			send_class[static_cast<size_t>(mv.second)] = send_before[static_cast<size_t>(mv.first)];
 			pending[static_cast<size_t>(mv.second)] = pending_before[static_cast<size_t>(mv.first)];
+			active[static_cast<size_t>(mv.second)] = active_before[static_cast<size_t>(mv.first)];
 		}
 		stream_of_lane.swap(next_sol);
 		for (const auto& mv : moves) {
@@ -1123,11 +1179,11 @@ struct oalsfx_engine {
 			for (int l = t * kLanes; l < (t + 1) * kLanes && mate < 0; ++l) {
 				mate = stream_of_lane[static_cast<size_t>(l)] >= 0 ? l : -1;
 			}
-			const bool active = mate >= 0;
+			const bool occupied = mate >= 0;
 			const bool changed = refill_padding || touched[static_cast<size_t>(t)] || !tile_active[static_cast<size_t>(t)] ||
 				!(tile_key[static_cast<size_t>(t)] == keys[static_cast<size_t>(std::max(k, 0))]);
-			tile_active[static_cast<size_t>(t)] = active ? 1 : 0;
-			if (!active) {
+			tile_active[static_cast<size_t>(t)] = occupied ? 1 : 0;
+			if (!occupied) {
 				continue;
 			}
 			const GroupKey& key = keys[static_cast<size_t>(k)];
@@ -1141,6 +1197,7 @@ struct oalsfx_engine {
 				}
 				send_class[static_cast<size_t>(l)] = key.send;
 				pending[static_cast<size_t>(l)] = static_cast<uint8_t>(key.pending);
+				active[static_cast<size_t>(l)] = key.paused ? 0 : 1;
 				if (changed) {
 					pad_to.push_back(l);
 					pad_from.push_back(mate);
@@ -1162,8 +1219,14 @@ struct oalsfx_engine {
 				}
 			}
 		}
-		return grow(stream_of_lane_dev, stream_of_lane_cap, stream_of_lane.size()) &&
-			be->upload(stream_of_lane_dev, stream_of_lane.data(), stream_of_lane.size() * sizeof(int32_t), nullptr) && be->sync(nullptr);
+		std::vector<int32_t> lane_map(stream_of_lane);
+		for (size_t l = 0; l < lane_map.size(); ++l) {
+			if (lane_map[l] >= 0 && !active[l]) {
+				lane_map[l] = -2 - lane_map[l];
+			}
+		}
+		return grow(stream_of_lane_dev, stream_of_lane_cap, lane_map.size()) &&
+			be->upload(stream_of_lane_dev, lane_map.data(), lane_map.size() * sizeof(int32_t), nullptr) && be->sync(nullptr);
 	}
 
 	// Groups of a placed engine: the active tiles only, every one of them whole and of one key.  Each slot signature with
@@ -1178,7 +1241,7 @@ struct oalsfx_engine {
 		multi_kernel = -1;
 		std::map<GroupKey, std::vector<TileRef>> by_key;
 		for (int t = 0; t < arena_tiles; ++t) {
-			if (tile_active[static_cast<size_t>(t)]) {
+			if (tile_active[static_cast<size_t>(t)] && !tile_key[static_cast<size_t>(t)].paused) {
 				by_key[tile_key[static_cast<size_t>(t)]].push_back(TileRef{static_cast<uint32_t>(t), 0xFFFFFFFFU});
 			}
 		}
@@ -1781,6 +1844,7 @@ int oalsfx_engine_create(const oalsfx_engine_desc* desc, oalsfx_engine** out)
 	SendSettings aux[kMaxSlots] = {unit, unit, unit, unit};
 	e->send_class.assign(static_cast<size_t>(e->streams), e->send_class_for(unit, aux));
 	e->pending.assign(static_cast<size_t>(e->streams), 0);
+	e->active.assign(static_cast<size_t>(e->streams), 1);
 	*out = e;
 	return OALSFX_OK;
 }
@@ -1870,6 +1934,71 @@ int oalsfx_engine_set_sends(oalsfx_engine* e, int first_stream, int n_streams, c
 	const int id = e->send_class_for(d, a);
 	for (int s = first_stream; s < first_stream + n_streams; ++s) {
 		e->send_class[static_cast<size_t>(e->lane_of(s))] = id;
+	}
+	e->groups_dirty = true;
+	return OALSFX_OK;
+}
+
+int oalsfx_engine_set_active(oalsfx_engine* e, int first_stream, int n_streams, int active)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	if (first_stream < 0 || n_streams < 1 || first_stream + n_streams > e->streams) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "Stream range is out of range.");
+	}
+	e->quiesce();
+	const uint8_t flag = active ? 1 : 0;
+	for (int s = first_stream; s < first_stream + n_streams; ++s) {
+		uint8_t& cur = e->active[static_cast<size_t>(e->lane_of(s))];
+		if (cur != flag) {
+			cur = flag;
+			e->groups_dirty = true;   // (an engine whose flags do not change keeps its groups)
+		}
+	}
+	return OALSFX_OK;
+}
+
+int oalsfx_engine_reset_streams(oalsfx_engine* e, int first_stream, int n_streams)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	if (first_stream < 0 || n_streams < 1 || first_stream + n_streams > e->streams) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "Stream range is out of range.");
+	}
+	if (!e->quiesce()) {  // zeroing state a running mix may still be using
+		return e->fail(OALSFX_ERR_DEVICE, e->be->error());
+	}
+	// The streams' lanes, by tile (placed streams sit in any order).  Every slot of them is marked pending as the
+	// set_effect call that configured it did, so the next block that mixes them runs `update` on fresh state: a slot
+	// holding an effect, that is -- the null effect has no update and no state.
+	std::map<uint32_t, uint32_t> masks;
+	for (int s = first_stream; s < first_stream + n_streams; ++s) {
+		const int lane = e->lane_of(s);
+		masks[static_cast<uint32_t>(lane / kLanes)] |= 1U << (lane % kLanes);
+		for (int slot = 0; slot < e->slots; ++slot) {
+			if (e->classes[static_cast<size_t>(e->fx_class[slot][static_cast<size_t>(lane)])].type != kFxNull) {
+				e->pending[static_cast<size_t>(lane)] |= static_cast<uint8_t>(1U << slot);
+			}
+		}
+	}
+	std::vector<TileRef> reset;
+	for (const auto& tm : masks) {
+		reset.push_back(TileRef{tm.first, tm.second});
+	}
+	const int n = static_cast<int>(reset.size());
+	bool ok = true;
+	for (int slot = 0; slot < e->slots && ok; ++slot) {
+		ok = e->be->zero_lanes(e->slot_state[slot], static_cast<long long>(kSlotStateWords) * kLanes, kSlotStateWords, reset.data(), n, nullptr);
+		if (ok && e->ring_cap[slot] > 0) {
+			ok = e->be->zero_lanes(reinterpret_cast<uint32_t*>(e->ring[slot]), static_cast<long long>(e->ring_cap[slot]) * kLanes,
+				e->ring_cap[slot], reset.data(), n, nullptr);
+		}
+	}
+	ok = ok && e->be->zero_lanes(e->send_state, static_cast<long long>(kSendStateWords) * kLanes, kSendStateWords, reset.data(), n, nullptr);
+	if (!ok) {
+		return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 	}
 	e->groups_dirty = true;
 	return OALSFX_OK;
@@ -1966,7 +2095,7 @@ int oalsfx_engine_mix(oalsfx_engine* e, int frames, const float* src, float* dst
 					return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 				}
 				if (g.key.pending != 0) {
-					std::fill(e->pending.begin(), e->pending.end(), static_cast<uint8_t>(0));
+					e->clear_mixed_pending();
 					e->groups_dirty = true;
 					e->frames_since_update = 0;
 				}
@@ -2038,8 +2167,12 @@ int oalsfx_engine_mix(oalsfx_engine* e, int frames, const float* src, float* dst
 				io_ts, io_ls, io_fs, io_cs, cuda_stream)) {
 			return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 		}
+		if (!e->placed && e->paused_rows > 0 && !e->be->zero_rows(ddst + done * io_fs, io_ts, io_ls, io_fs, io_cs, e->paused_rows_dev,
+				e->paused_rows, todo, e->channels, cuda_stream)) {
+			return e->fail(OALSFX_ERR_DEVICE, e->be->error());
+		}
 		if (had_pending) {
-			std::fill(e->pending.begin(), e->pending.end(), static_cast<uint8_t>(0));
+			e->clear_mixed_pending();
 			e->groups_dirty = true;
 			e->frames_since_update = 0;
 		}

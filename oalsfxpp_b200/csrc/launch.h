@@ -20,13 +20,15 @@ bool launch_relay_family(int kernel_id, const MixArgs& args, cudaStream_t stream
 bool launch_span_family(int kernel_id, const MixArgs& args, cudaStream_t stream);     // k_span.cu: block-parallel in time
 bool launch_scan_family(int kernel_id, const MixArgs& args, cudaStream_t stream);     // k_scan.cu: linear-recurrence scan over time
 
-// k_place.cu: stream placement (see Backend::copy_lanes / gather_io / scatter_io)
+// k_place.cu: stream placement and paused streams (see Backend::copy_lanes / gather_io / scatter_io / zero_rows)
 bool launch_copy_lanes(uint32_t* dst, long long dst_ts, int dst_w0, const uint32_t* src, long long src_ts, int src_w0, int words,
 	const int32_t* from, const int32_t* to, int n, cudaStream_t stream);
 bool launch_gather_io(const float* src, long long ts, long long ls, long long fs, long long cs, const int32_t* stream_of_lane,
 	int lane_tiles, int frames, int channels, float* dst, cudaStream_t stream);
 bool launch_scatter_io(const float* src, const int32_t* stream_of_lane, int lane_tiles, int frames, int channels, float* dst,
 	long long ts, long long ls, long long fs, long long cs, cudaStream_t stream);
+bool launch_zero_rows(float* dst, long long ts, long long ls, long long fs, long long cs, const int32_t* rows, int n, int frames,
+	int channels, cudaStream_t stream);
 
 // Shared-memory carve-out of a kernel, set once.  Tuning knobs (experiments only): OALSFX_TUNE_CARVEOUT = percent or
 // -1 (driver default), OALSFX_TUNE_DYN_SMEM = bytes of unused dynamic shared memory per CTA (caps residency).

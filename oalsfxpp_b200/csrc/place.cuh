@@ -7,7 +7,9 @@
 //                       tile-mate's state; a snapshot gathers the caller streams into canonical order.
 //   gather_io_kernel  : the caller's sample buffer (either layout, four strides) -> an engine-internal TILED block in
 //                       lane order, zeros for padding lanes.
-//   scatter_io_kernel : the reverse, writing the caller rows only.
+//   scatter_io_kernel : the reverse, writing the caller rows only.  A parked lane (a paused stream s, encoded in the lane
+//                       map as -2 - s: the gather treats it as absent) receives zeros in its caller row instead.
+//   zero_rows_kernel  : zeros in the caller rows of a list of streams: the paused streams of an unplaced engine.
 // The mix kernels then run unchanged on the TILED block.  copy_lane_word is the element body the kernel and the host loop
 // share; the host loops (the Backend defaults, backend.h) serve the CPU test backend, the kernels the device.
 #ifndef OALSFX_PLACE_CUH
@@ -69,15 +71,28 @@ inline void scatter_io_host(const float* src, const int32_t* stream_of_lane, int
 	long long ts, long long ls, long long fs, long long cs)
 {
 	for (long long l = 0; l < static_cast<long long>(lane_tiles) * kLanes; ++l) {
-		const int s = stream_of_lane[l];
+		const int m = stream_of_lane[l];
+		const int s = m >= 0 ? m : -2 - m;   // (m == -1: padding lane, s < 0)
 		for (int f = 0; s >= 0 && f < frames; ++f) {
 			for (int c = 0; c < channels; ++c) {
-				dst[(s / kLanes) * ts + (s % kLanes) * ls + f * fs + c * cs] = src[tiled_index(l, f, c, frames, channels)];
+				dst[(s / kLanes) * ts + (s % kLanes) * ls + f * fs + c * cs] = m >= 0 ? src[tiled_index(l, f, c, frames, channels)] : 0.0F;
 			}
 		}
 	}
 }
 
+inline void zero_rows_host(float* dst, long long ts, long long ls, long long fs, long long cs, const int32_t* rows, int n, int frames,
+	int channels)
+{
+	for (int i = 0; i < n; ++i) {
+		const int s = rows[i];
+		for (int f = 0; f < frames; ++f) {
+			for (int c = 0; c < channels; ++c) {
+				dst[(s / kLanes) * ts + (s % kLanes) * ls + f * fs + c * cs] = 0.0F;
+			}
+		}
+	}
+}
 
 } // namespace place
 } // namespace oalsfx

@@ -51,6 +51,10 @@ def bind(lib):
     lib.oalsfx_engine_set_effect.restype = i32
     lib.oalsfx_engine_set_sends.argtypes = [vp, i32, i32, f32p, f32p]
     lib.oalsfx_engine_set_sends.restype = i32
+    lib.oalsfx_engine_set_active.argtypes = [vp, i32, i32, i32]
+    lib.oalsfx_engine_set_active.restype = i32
+    lib.oalsfx_engine_reset_streams.argtypes = [vp, i32, i32]
+    lib.oalsfx_engine_reset_streams.restype = i32
     lib.oalsfx_engine_mix.argtypes = [vp, i32, vp, vp, i32, i32, vp]
     lib.oalsfx_engine_mix.restype = i32
     lib.oalsfx_engine_pin_host.argtypes = [vp, vp, C.c_size_t]
@@ -104,7 +108,7 @@ def bind(lib):
 
 EXPORTED_SYMBOLS = (
     "oalsfx_engine_create", "oalsfx_engine_destroy", "oalsfx_engine_set_effect",
-    "oalsfx_engine_set_sends", "oalsfx_engine_mix", "oalsfx_engine_mix_bus", "oalsfx_engine_reduce_bus",
+    "oalsfx_engine_set_sends", "oalsfx_engine_set_active", "oalsfx_engine_reset_streams", "oalsfx_engine_mix", "oalsfx_engine_mix_bus", "oalsfx_engine_reduce_bus",
     "oalsfx_engine_pin_host", "oalsfx_engine_unpin_host",
     "oalsfx_engine_debug_state", "oalsfx_debug_waveshaper", "oalsfx_plan_placement", "oalsfx_engine_launch_count", "oalsfx_engine_last_kernel", "oalsfx_engine_device_bytes",
     "oalsfx_last_error", "oalsfx_build_info", "oalsfx_effect_defaults", "oalsfx_effect_normalize",
@@ -220,6 +224,17 @@ class Engine:
         flat = [v for triple in aux for v in triple]
         a = (C.c_float * len(flat))(*flat)
         self._check(self.lib.oalsfx_engine_set_sends(self._h, first_stream, n, d, a))
+
+    def set_active(self, active, first_stream=0, n_streams=None):
+        """Mix (True) or pause (False) the stream range.  A paused stream keeps all of its state, its input is not read and
+        its output rows are zeros; it resumes bit for bit where it stopped."""
+        n = self.num_streams - first_stream if n_streams is None else n_streams
+        self._check(self.lib.oalsfx_engine_set_active(self._h, first_stream, n, 1 if active else 0))
+
+    def reset(self, first_stream=0, n_streams=None):
+        """The stream range restarts from silence with its current effects and sends, like a freshly created engine."""
+        n = self.num_streams - first_stream if n_streams is None else n_streams
+        self._check(self.lib.oalsfx_engine_reset_streams(self._h, first_stream, n))
 
     def mix(self, src, dst=None, frames=None, layout=LAYOUT_STREAM_MAJOR, space=None, stream=0):
         """Api::mix for every stream.  numpy arrays are host buffers, torch CUDA tensors device buffers."""
