@@ -129,6 +129,36 @@ int oalsfx_engine_unpin_host(oalsfx_engine* e, void* buffer);
 int oalsfx_engine_mix_bus(oalsfx_engine* e, int frames, const float* src, float* dst, int layout,
 	float* bus, void* cuda_stream);
 
+/* Submix buses.  A host sums its voices into a few buses -- per listener, player, room or category -- rather than
+ * consuming one output row per stream.  Every stream is routed to one bus (>= 0) or to none (OALSFX_BUS_NONE); a new
+ * engine routes every stream to bus 0.  Routing is configuration, like effect types and activity: reset_streams and
+ * set_placement keep it, snapshots do not hold it and restore leaves it alone.
+ * oalsfx_engine_route_streams: bus[i] becomes the bus of stream first_stream + i.  Waits for the stream the caller last
+ * passed in, as set_active does; OALSFX_ERR_ARGUMENT for a bad range, a null `bus` or an entry below OALSFX_BUS_NONE.
+ * oalsfx_engine_reduce_buses: buses[(b * frames + f) * C + c] (DEVICE array of n_buses * frames * C floats) = the sum over
+ * the members of bus b of a device buffer `dst` produced by oalsfx_engine_mix (either layout).  The members of bus b are
+ * the streams routed to b that are active at the time of the call (paused streams are not members and their rows are
+ * not read; padding lanes of TILED buffers never are).  Every one of the n_buses buses is written; a bus without
+ * members receives +0.0f.  Summation order, the same for every (frame, channel):
+ *   - the members of the bus in ascending caller stream index are the level-0 list;
+ *   - while the list has more than one entry, it is cut into consecutive runs of 32 (the last one shorter); each run is
+ *     summed left to right in fp32 starting from +0.0f; the run sums, in order, are the next level's list;
+ *   - a single member gives +0.0f + v.
+ * The order depends neither on the layout nor on the placement mode nor on how the frames of a call are processed, so
+ * STREAM_MAJOR and TILED give bit-identical buses, so do CALLER and AUTO placement, and one call of many frames equals
+ * one call per block.  (The all-streams bus of oalsfx_engine_reduce_bus keeps its own order.)  OALSFX_ERR_ARGUMENT for a
+ * null pointer, frames <= 0, an unknown layout, n_buses < 1 or n_buses not above every routed bus index.  Enqueued on
+ * `cuda_stream`, returns at once; after a routing or activity change the first call rebuilds and uploads the bus plan,
+ * the others neither synchronize, allocate nor upload.  With several GPUs each rank's buses sum with one all-reduce.
+ * oalsfx_engine_mix_buses: oalsfx_engine_mix (device buffers) and oalsfx_engine_reduce_buses on the same stream; every
+ * argument is checked before the mix, so a refused call advances no stream. */
+enum { OALSFX_BUS_NONE = -1 };
+int oalsfx_engine_route_streams(oalsfx_engine* e, int first_stream, int n_streams, const int32_t* bus);
+int oalsfx_engine_reduce_buses(oalsfx_engine* e, int frames, const float* dst, int layout,
+	int n_buses, float* buses, void* cuda_stream);
+int oalsfx_engine_mix_buses(oalsfx_engine* e, int frames, const float* src, float* dst, int layout,
+	int n_buses, float* buses, void* cuda_stream);
+
 /* PCM formats either side of the path (device buffers; SURVEY.md 8f rank 2).  The reference's only
  * producer and consumer of Api::mix buffers is its WAV demo, and these are its conversions:
  *   oalsfx_pcm_to_float : bit_depth 8: (u8 - 128) / 128.0f, 16: s16 / 32768.0f  (oalsfxpp_test.cpp:703-740)

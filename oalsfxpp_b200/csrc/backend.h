@@ -12,6 +12,7 @@
 #include <cstdint>
 #include <string>
 
+#include "bus.cuh"
 #include "mix.cuh"
 #include "place.cuh"
 
@@ -80,6 +81,14 @@ public:
 	// bus[frame*C + c] = sum over streams (fixed order: lane-major tree per tile, then tiles).
 	virtual bool reduce_bus(const float* data, long long ts, long long ls, long long fs, long long cs,
 		int num_streams, int frames, int channels, float* bus, void* stream) = 0;
+	// Submix buses (bus.cuh): every level of one chunk of frames, in level order; plan and scratch are device memory.  The
+	// default is bus.cuh's host loop over the kernels' element body, for the CPU test backend; cuda_backend.cu overrides it
+	// with the sm_100a kernels of k_bus.cu.
+	virtual bool reduce_buses(const bus::Chunk& chunk, void*)
+	{
+		bus::reduce_buses_host(chunk);
+		return true;
+	}
 	// PCM formats either side of the path (SURVEY.md 8f rank 2; the reference's only producer/consumer of
 	// sample buffers, its WAV demo: oalsfxpp_test.cpp:703-740 ingest, :602-651 egress).  Device pointers.
 	//   pcm_to_float : bits = 8  -> (int(u8) - 128) / 128.0f ;  bits = 16 -> s16 / 32768.0f

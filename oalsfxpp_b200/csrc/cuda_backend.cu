@@ -469,6 +469,13 @@ public:
 		return check(cudaGetLastError(), "reduce_bus_kernel");
 	}
 
+	bool reduce_buses(const bus::Chunk& chunk, void* stream) override
+	{
+		DeviceScope scope(this);
+		return scope.ok && launch_reduce_buses(chunk, static_cast<cudaStream_t>(stream)) &&
+			check(cudaGetLastError(), "bus_rows_kernel / bus_tiled_kernel");
+	}
+
 	bool pcm_to_float(const void* src, int bits, float* dst, long long count, void* stream) override
 	{
 		DeviceScope scope(this);

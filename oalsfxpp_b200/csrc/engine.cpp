@@ -167,6 +167,24 @@ struct oalsfx_engine {
 	int lane_count() const { return placed ? arena_tiles * kLanes : streams; }
 	int lane_of(int s) const { return placed ? lane_of_stream[static_cast<size_t>(s)] : s; }
 
+	// Submix buses (oalsfx_engine_route_streams / reduce_buses, bus.cuh).  The routing is kept in caller order; the plan --
+	// the members of every bus (its active streams, ascending) and the runs of every level of the summation tree -- depends
+	// on caller streams and activity only, is rebuilt on the host at the first reduce after a routing or activity change
+	// and uploaded once.  Lane moves do not touch it.
+	std::vector<int32_t> bus_of_stream;  // OALSFX_BUS_NONE (-1) or a bus index, per caller stream
+	int max_bus = 0;                     // largest bus index any stream is routed to (-1: none)
+	bool bus_plan_dirty = true;
+	std::vector<int32_t> bus_plan;       // host image of bus_plan_dev: the member list, then every level's runs
+	int bus_levels = 0;
+	size_t bus_run_word[bus::kBusMaxLevels] = {};       // word offset of the level's runs in the plan
+	int bus_runs[bus::kBusMaxLevels] = {};
+	long long bus_partial_row[bus::kBusMaxLevels] = {}; // first scratch row of the level's partial rows
+	long long bus_partial_rows = 0;
+	int32_t* bus_plan_dev = nullptr;
+	size_t bus_plan_cap = 0;            // words
+	float* bus_scratch = nullptr;       // partial rows of one chunk (<= kBusChunkFrames frames)
+	size_t bus_scratch_cap = 0;         // floats
+
 	std::vector<Group> groups;
 	// Class-per-tile launch (duo_multi_kernel): the class table and every tile's class index in HBM; `groups` is
 	// then the single multi group and `fallback_groups` holds the per-class / table-mode groups for the blocks the
@@ -269,6 +287,8 @@ struct oalsfx_engine {
 		be->release(move_scratch);
 		be->release(io_in);
 		be->release(io_out);
+		be->release(bus_plan_dev);
+		be->release(bus_scratch);
 		be->stream_destroy(pipe_in);
 		be->stream_destroy(pipe_run);
 		be->stream_destroy(pipe_out);
@@ -519,6 +539,154 @@ struct oalsfx_engine {
 		k.pending = pending[static_cast<size_t>(s)];
 		k.paused = active[static_cast<size_t>(s)] ? 0U : 1U;
 		return k;
+	}
+
+	// ---- submix buses ------------------------------------------------------------------------------
+	// The reason a reduce_buses / mix_buses call is refused, checked before anything runs, or null.
+	const char* bad_bus_args(int frames, const float* dst, int layout, int n_buses, const float* buses) const
+	{
+		if (!dst || !buses) {
+			return "No block or bus buffer.";
+		}
+		if (frames <= 0) {
+			return "Frame count must be positive.";
+		}
+		if (layout != OALSFX_LAYOUT_STREAM_MAJOR && layout != OALSFX_LAYOUT_TILED) {
+			return "Unknown layout.";
+		}
+		if (n_buses < 1 || n_buses <= max_bus) {
+			return "n_buses must be at least 1 and above every bus index a stream is routed to.";
+		}
+		return nullptr;
+	}
+
+	// Members of every bus 0..max_bus in CSR order, then level by level: a bus whose list has one run left ends in that
+	// run (it writes the bus row), every other bus cuts its list into runs of 32 that write partial rows, which are the
+	// bus's list at the next level.
+	bool rebuild_bus_plan(void* stream)
+	{
+		const int nb = max_bus + 1;
+		std::vector<int32_t> start(static_cast<size_t>(nb) + 1, 0);
+		for (int s = 0; s < streams; ++s) {
+			const int b = bus_of_stream[static_cast<size_t>(s)];
+			if (b >= 0 && active[static_cast<size_t>(lane_of(s))]) {
+				++start[static_cast<size_t>(b) + 1];
+			}
+		}
+		for (int b = 0; b < nb; ++b) {
+			start[static_cast<size_t>(b) + 1] += start[static_cast<size_t>(b)];
+		}
+		bus_plan.assign(static_cast<size_t>(start[static_cast<size_t>(nb)]), 0);
+		std::vector<int32_t> fill(start.begin(), start.end() - 1);
+		for (int s = 0; s < streams; ++s) {
+			const int b = bus_of_stream[static_cast<size_t>(s)];
+			if (b >= 0 && active[static_cast<size_t>(lane_of(s))]) {
+				bus_plan[static_cast<size_t>(fill[static_cast<size_t>(b)]++)] = s;
+			}
+		}
+		struct List {
+			int bus;
+			int32_t src, len;
+		};
+		std::vector<List> open, next;
+		for (int b = 0; b < nb; ++b) {
+			open.push_back(List{b, start[static_cast<size_t>(b)], start[static_cast<size_t>(b) + 1] - start[static_cast<size_t>(b)]});
+		}
+		bus_levels = 0;
+		bus_partial_rows = 0;
+		while (!open.empty()) {
+			const int level = bus_levels++;
+			bus_run_word[level] = bus_plan.size();
+			bus_partial_row[level] = bus_partial_rows;
+			int32_t partials = 0;
+			next.clear();
+			for (const List& l : open) {
+				const int32_t n_runs = std::max<int32_t>(1, (l.len + bus::kBusRun - 1) / bus::kBusRun);
+				if (n_runs == 1) {
+					bus_plan.insert(bus_plan.end(), {l.src, l.len, -1 - l.bus});
+					continue;
+				}
+				next.push_back(List{l.bus, partials, n_runs});
+				for (int32_t r = 0; r < n_runs; ++r) {
+					bus_plan.insert(bus_plan.end(), {l.src + r * bus::kBusRun, std::min<int32_t>(bus::kBusRun, l.len - r * bus::kBusRun), partials++});
+				}
+			}
+			bus_runs[level] = static_cast<int>((bus_plan.size() - bus_run_word[level]) / 3);
+			bus_partial_rows += partials;
+			open.swap(next);
+		}
+		if (bus_plan.size() > bus_plan_cap) {
+			quiesce();   // a reduce may still read the old plan
+			be->release(bus_plan_dev);
+			device_bytes -= static_cast<long long>(bus_plan_cap * sizeof(int32_t));
+			bus_plan_cap = 0;
+			bus_plan_dev = static_cast<int32_t*>(dev_alloc(bus_plan.size() * sizeof(int32_t)));
+			if (!bus_plan_dev) {
+				return false;
+			}
+			bus_plan_cap = bus_plan.size();
+		}
+		if (!bus_plan.empty() && !be->upload(bus_plan_dev, bus_plan.data(), bus_plan.size() * sizeof(int32_t), stream)) {
+			return false;
+		}
+		bus_plan_dirty = false;
+		return true;
+	}
+
+	// oalsfx_engine_reduce_buses with checked arguments: chunks of <= kBusChunkFrames frames, one launch per level each;
+	// buses above every routed index have no members and are zeroed.
+	int reduce_buses(int frames, const float* dst, int layout, int n_buses, float* buses, void* stream)
+	{
+		note_stream(stream);
+		if (bus_plan_dirty && !rebuild_bus_plan(stream)) {
+			return fail(OALSFX_ERR_DEVICE, "Bus plan upload failed: " + be->error());
+		}
+		const int chunk = std::min(frames, bus::kBusChunkFrames);
+		const size_t need = static_cast<size_t>(bus_partial_rows) * static_cast<size_t>(chunk) * static_cast<size_t>(channels);
+		if (need > bus_scratch_cap) {
+			quiesce();
+			be->release(bus_scratch);
+			device_bytes -= static_cast<long long>(bus_scratch_cap * sizeof(float));
+			bus_scratch_cap = 0;
+			bus_scratch = static_cast<float*>(dev_alloc(need * sizeof(float)));
+			if (!bus_scratch) {
+				return fail(OALSFX_ERR_MEMORY, "Bus scratch allocation failed: " + be->error());
+			}
+			bus_scratch_cap = need;
+		}
+		bus::Chunk k;
+		std::memset(&k, 0, sizeof(k));
+		k.dst = dst;
+		k.ts = static_cast<long long>(frames) * channels * kLanes;
+		k.ls = layout == OALSFX_LAYOUT_TILED ? 1 : static_cast<long long>(frames) * channels;
+		k.fs = layout == OALSFX_LAYOUT_TILED ? static_cast<long long>(channels) * kLanes : channels;
+		k.cs = layout == OALSFX_LAYOUT_TILED ? kLanes : 1;
+		k.frames = frames;
+		k.channels = channels;
+		k.members = bus_plan_dev;
+		k.levels = bus_levels;
+		k.buses = buses;
+		for (int level = 0; level < bus_levels; ++level) {
+			k.runs[level] = reinterpret_cast<const bus::Run*>(bus_plan_dev + bus_run_word[level]);
+			k.n_runs[level] = bus_runs[level];
+		}
+		for (int f0 = 0; f0 < frames; f0 += bus::kBusChunkFrames) {
+			k.f0 = f0;
+			k.nf = std::min(frames - f0, bus::kBusChunkFrames);
+			for (int level = 0; level < bus_levels; ++level) {
+				k.partial[level] = bus_scratch ? bus_scratch + bus_partial_row[level] * k.nf * channels : nullptr;
+			}
+			launches += bus_levels;
+			if (!be->reduce_buses(k, stream)) {
+				return fail(OALSFX_ERR_DEVICE, be->error());
+			}
+		}
+		const long long per_bus = static_cast<long long>(frames) * channels;
+		if (n_buses > max_bus + 1 && !be->zero(buses + (max_bus + 1) * per_bus,
+				static_cast<size_t>(n_buses - max_bus - 1) * static_cast<size_t>(per_bus) * sizeof(float), stream)) {
+			return fail(OALSFX_ERR_DEVICE, be->error());
+		}
+		return OALSFX_OK;
 	}
 
 	// After a block that consumed updates: the lanes that were mixed have none left; paused lanes keep theirs for the
@@ -1845,6 +2013,7 @@ int oalsfx_engine_create(const oalsfx_engine_desc* desc, oalsfx_engine** out)
 	e->send_class.assign(static_cast<size_t>(e->streams), e->send_class_for(unit, aux));
 	e->pending.assign(static_cast<size_t>(e->streams), 0);
 	e->active.assign(static_cast<size_t>(e->streams), 1);
+	e->bus_of_stream.assign(static_cast<size_t>(e->streams), 0);
 	*out = e;
 	return OALSFX_OK;
 }
@@ -1954,6 +2123,7 @@ int oalsfx_engine_set_active(oalsfx_engine* e, int first_stream, int n_streams, 
 		if (cur != flag) {
 			cur = flag;
 			e->groups_dirty = true;   // (an engine whose flags do not change keeps its groups)
+			e->bus_plan_dirty = true;
 		}
 	}
 	return OALSFX_OK;
@@ -2001,6 +2171,33 @@ int oalsfx_engine_reset_streams(oalsfx_engine* e, int first_stream, int n_stream
 		return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 	}
 	e->groups_dirty = true;
+	return OALSFX_OK;
+}
+
+int oalsfx_engine_route_streams(oalsfx_engine* e, int first_stream, int n_streams, const int32_t* bus)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	if (first_stream < 0 || n_streams < 1 || first_stream + n_streams > e->streams || !bus) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "Bad stream range or null bus list.");
+	}
+	for (int i = 0; i < n_streams; ++i) {
+		if (bus[i] < OALSFX_BUS_NONE) {
+			return e->fail(OALSFX_ERR_ARGUMENT, "Bus index below OALSFX_BUS_NONE.");
+		}
+	}
+	e->quiesce();
+	bool changed = false;
+	for (int i = 0; i < n_streams; ++i) {
+		int32_t& cur = e->bus_of_stream[static_cast<size_t>(first_stream + i)];
+		changed = changed || cur != bus[i];
+		cur = bus[i];
+	}
+	if (changed) {
+		e->max_bus = *std::max_element(e->bus_of_stream.begin(), e->bus_of_stream.end());
+		e->bus_plan_dirty = true;
+	}
 	return OALSFX_OK;
 }
 
@@ -2249,6 +2446,34 @@ int oalsfx_engine_reduce_bus(oalsfx_engine* e, int frames, const float* dst, int
 		return e->fail(OALSFX_ERR_DEVICE, e->be->error());
 	}
 	return OALSFX_OK;
+}
+
+int oalsfx_engine_reduce_buses(oalsfx_engine* e, int frames, const float* dst, int layout, int n_buses, float* buses, void* cuda_stream)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	if (const char* bad = e->bad_bus_args(frames, dst, layout, n_buses, buses)) {
+		return e->fail(OALSFX_ERR_ARGUMENT, bad);
+	}
+	return e->reduce_buses(frames, dst, layout, n_buses, buses, cuda_stream);
+}
+
+int oalsfx_engine_mix_buses(oalsfx_engine* e, int frames, const float* src, float* dst, int layout, int n_buses, float* buses,
+	void* cuda_stream)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	// everything is checked before the mix: a refused call advances no stream
+	if (!src) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "No source samples.");
+	}
+	if (const char* bad = e->bad_bus_args(frames, dst, layout, n_buses, buses)) {
+		return e->fail(OALSFX_ERR_ARGUMENT, bad);
+	}
+	const int rc = oalsfx_engine_mix(e, frames, src, dst, layout, OALSFX_SPACE_DEVICE, cuda_stream);
+	return rc != OALSFX_OK ? rc : e->reduce_buses(frames, dst, layout, n_buses, buses, cuda_stream);
 }
 
 int oalsfx_pcm_to_float(oalsfx_engine* e, const void* src, int bit_depth, float* dst, long long count, void* cuda_stream)

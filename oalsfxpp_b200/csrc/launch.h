@@ -9,6 +9,7 @@
 
 #include <cstdlib>
 
+#include "bus.cuh"
 #include "kernel_table.h"
 
 namespace oalsfx {
@@ -29,6 +30,8 @@ bool launch_scatter_io(const float* src, const int32_t* stream_of_lane, int lane
 	long long ts, long long ls, long long fs, long long cs, cudaStream_t stream);
 bool launch_zero_rows(float* dst, long long ts, long long ls, long long fs, long long cs, const int32_t* rows, int n, int frames,
 	int channels, cudaStream_t stream);
+// k_bus.cu: every level of one chunk of the submix buses (see Backend::reduce_buses)
+bool launch_reduce_buses(const bus::Chunk& chunk, cudaStream_t stream);
 
 // Shared-memory carve-out of a kernel, set once.  Tuning knobs (experiments only): OALSFX_TUNE_CARVEOUT = percent or
 // -1 (driver default), OALSFX_TUNE_DYN_SMEM = bytes of unused dynamic shared memory per CTA (caps residency).

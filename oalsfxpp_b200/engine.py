@@ -15,6 +15,7 @@ from .props import EffectProps, EffectType, channel_count
 
 LAYOUT_STREAM_MAJOR = 0
 LAYOUT_TILED = 1
+BUS_NONE = -1
 SPACE_HOST = 0
 SPACE_DEVICE = 1
 
@@ -65,6 +66,12 @@ def bind(lib):
     lib.oalsfx_engine_mix_bus.restype = i32
     lib.oalsfx_engine_reduce_bus.argtypes = [vp, i32, vp, i32, vp, vp]
     lib.oalsfx_engine_reduce_bus.restype = i32
+    lib.oalsfx_engine_route_streams.argtypes = [vp, i32, i32, vp]
+    lib.oalsfx_engine_route_streams.restype = i32
+    lib.oalsfx_engine_reduce_buses.argtypes = [vp, i32, vp, i32, i32, vp, vp]
+    lib.oalsfx_engine_reduce_buses.restype = i32
+    lib.oalsfx_engine_mix_buses.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp]
+    lib.oalsfx_engine_mix_buses.restype = i32
     lib.oalsfx_engine_debug_state.argtypes = [vp, i32, i32, C.POINTER(C.c_int32)]
     lib.oalsfx_engine_debug_state.restype = i32
     lib.oalsfx_engine_launch_count.argtypes = [vp]
@@ -109,6 +116,7 @@ def bind(lib):
 EXPORTED_SYMBOLS = (
     "oalsfx_engine_create", "oalsfx_engine_destroy", "oalsfx_engine_set_effect",
     "oalsfx_engine_set_sends", "oalsfx_engine_set_active", "oalsfx_engine_reset_streams", "oalsfx_engine_mix", "oalsfx_engine_mix_bus", "oalsfx_engine_reduce_bus",
+    "oalsfx_engine_route_streams", "oalsfx_engine_reduce_buses", "oalsfx_engine_mix_buses",
     "oalsfx_engine_pin_host", "oalsfx_engine_unpin_host",
     "oalsfx_engine_debug_state", "oalsfx_debug_waveshaper", "oalsfx_plan_placement", "oalsfx_engine_launch_count", "oalsfx_engine_last_kernel", "oalsfx_engine_device_bytes",
     "oalsfx_last_error", "oalsfx_build_info", "oalsfx_effect_defaults", "oalsfx_effect_normalize",
@@ -272,6 +280,33 @@ class Engine:
         self._check(self.lib.oalsfx_engine_reduce_bus(self._h, int(frames), _ptr(dst), layout, _ptr(bus),
                                                       C.c_void_p(stream)))
         return bus
+
+    def route(self, bus, first_stream=0):
+        """Route streams first_stream, first_stream + 1, ... to the buses in `bus` (ints; BUS_NONE = -1: no bus)."""
+        bus = np.ascontiguousarray(bus, dtype=np.int32).ravel()
+        self._check(self.lib.oalsfx_engine_route_streams(self._h, int(first_stream), int(bus.size), bus.ctypes.data))
+
+    def _bus_count(self, frames, buses, n_buses):
+        if n_buses is not None:
+            return int(n_buses)
+        size = buses.size if isinstance(buses, np.ndarray) else buses.numel() if hasattr(buses, "numel") else None
+        if size is None:
+            raise ValueError("n_buses is required for raw pointers")
+        return size // (int(frames) * self.channels)
+
+    def reduce_buses(self, frames, dst, buses, layout=LAYOUT_STREAM_MAJOR, stream=0, n_buses=None):
+        """buses ([n_buses][frames][channels], device) = per bus the sum of the rows of `dst` (device, as mix() wrote it) of
+        the active streams routed to it, in the fixed order of include/oalsfx_engine.h.  n_buses defaults to the size of
+        `buses`."""
+        self._check(self.lib.oalsfx_engine_reduce_buses(self._h, int(frames), _ptr(dst), layout,
+                                                        self._bus_count(frames, buses, n_buses), _ptr(buses), C.c_void_p(stream)))
+        return buses
+
+    def mix_buses(self, src, dst, frames, buses, layout=LAYOUT_STREAM_MAJOR, stream=0, n_buses=None):
+        """mix() on device buffers followed by reduce_buses() of its output on the same stream."""
+        self._check(self.lib.oalsfx_engine_mix_buses(self._h, int(frames), _ptr(src), _ptr(dst), layout,
+                                                     self._bus_count(frames, buses, n_buses), _ptr(buses), C.c_void_p(stream)))
+        return buses
 
     def debug_state(self, stream, slot):
         out = (C.c_int32 * 4)()
