@@ -154,6 +154,44 @@ int oalsfx_engine_mix_bus(oalsfx_engine* e, int frames, const float* src, float*
  * argument is checked before the mix, so a refused call advances no stream. */
 enum { OALSFX_BUS_NONE = -1 };
 int oalsfx_engine_route_streams(oalsfx_engine* e, int first_stream, int n_streams, const int32_t* bus);
+
+/* Routes with gains.  A stream may feed up to OALSFX_MAX_ROUTES buses -- its category bus and a room's reverb send, one bus
+ * per listener in split screen, two rooms while a voice moves between them -- each route with its own gain, and a gain
+ * change ramps over a given number of frames instead of jumping (the reference ramps every gain it changes: MixHelpers
+ * gain steps, oalsfxpp.cpp:2762-2797).
+ * oalsfx_engine_set_routes: with R = routes_per_stream (1..OALSFX_MAX_ROUTES), the routes of stream first_stream + i
+ * become the entries r < R with bus[i * R + r] != OALSFX_BUS_NONE, each with gain gain[i * R + r] (gain NULL: 1.0f);
+ * every other route of the stream is removed.  OALSFX_ERR_ARGUMENT, with nothing changed, for a bad range, R outside
+ * 1..OALSFX_MAX_ROUTES, a null `bus`, a bus index below OALSFX_BUS_NONE, a stream naming the same bus twice, a gain that is
+ * not finite, or ramp_frames outside [0, 2^24].  Waits for the stream the caller last passed in, as route_streams does.
+ * oalsfx_engine_route_streams(e, first, n, bus) is set_routes(e, first, n, 1, bus, NULL, 0): it also removes a stream's
+ * other routes.  Routes and ramps in progress are configuration like the routing: reset_streams, set_placement and
+ * restore keep them, snapshots do not hold them.  In reduce_buses / mix_buses n_buses must be above every bus any route
+ * names.
+ *   - The frame clock: the engine counts the frames it has mixed; every successful mix / mix_bus / mix_buses call adds its
+ *     `frames`, whichever streams are paused and whichever space its buffers are in (a refused call adds nothing).  M is
+ *     the clock at the start of the most recent such call (0 before the first), and reduce_buses gives frame f of its
+ *     block the clock value T = M + f.  So reduce_buses right after mix equals mix_buses, reducing a block twice or in
+ *     both layouts gives the same bits, and one long call equals one call per block.
+ *   - A route holds a start gain g0, a target gain g1, a ramp length Rf and a ramp start T0.  Its gain at clock T, in fp32
+ *     with one rounding per operation, in this order, no contraction:  T < T0: g0;  Rf == 0 or T - T0 >= Rf: g1;
+ *     otherwise g0 + (g1 - g0) * ((float)(T - T0 + 1) / (float)Rf).
+ *   - set_routes(..., ramp_frames) sets, for every route it lists: T0 = the clock now (the first frame of the next mix),
+ *     Rf = ramp_frames, g1 = the new gain, and g0 = the route's gain at T0 - 1 when the stream already had a route to that
+ *     bus (the gain its last mixed frame received, or its old g0 if nothing was mixed since the last change), else 0.0f.
+ *     With ramp_frames == 0, g0 = g1: the new gain holds at every T, so a block mixed before the call is reduced with it,
+ *     as route_streams has always done.
+ *     A crossfade between rooms is therefore one call, {old: 0, new: 1} with a ramp, and once the ramp has ended
+ *     {new: 1}.  A removed route stops at once: ramp it to 0 first.
+ *   - Bus b's members are the routes to b of the streams active at the call, in ascending caller stream index (a stream
+ *     has at most one route per bus); a member's value is the fp32 product gain(T) * x, one rounding, and the members are
+ *     summed in the order above.  Routes of gain 0 are members (0 * Inf is NaN on the bus).  A chunk of frames in which
+ *     every member's gain is 1.0f runs the unweighted sum, which gives the same bits at the speed of plain routing.
+ *   - A call that changes gains or ramps only, keeping every (stream, bus) pair, costs one upload of the gains at the next
+ *     reduce; a change of the pairs rebuilds the bus plan as route_streams does. */
+enum { OALSFX_MAX_ROUTES = 4 };
+int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream,
+	const int32_t* bus, const float* gain, int ramp_frames);
 int oalsfx_engine_reduce_buses(oalsfx_engine* e, int frames, const float* dst, int layout,
 	int n_buses, float* buses, void* cuda_stream);
 int oalsfx_engine_mix_buses(oalsfx_engine* e, int frames, const float* src, float* dst, int layout,

@@ -8,12 +8,12 @@ processing of its own and there is no CPU fallback: importing works anywhere, bu
 """
 from .props import (ChannelFormat, EffectType, EffectProps, channel_count, default_props,
                     normalize_props, reverb_preset, reverb_preset_names)
-from .engine import (Engine, OalsfxError, LAYOUT_STREAM_MAJOR, LAYOUT_TILED, BUS_NONE, SPACE_HOST,
+from .engine import (Engine, OalsfxError, LAYOUT_STREAM_MAJOR, LAYOUT_TILED, BUS_NONE, MAX_ROUTES, SPACE_HOST,
                      SPACE_DEVICE, library_path, load_library, build_info, plan_placement)
 
 __all__ = [
     "ChannelFormat", "EffectType", "EffectProps", "channel_count", "default_props",
     "normalize_props", "reverb_preset", "reverb_preset_names", "Engine", "OalsfxError",
-    "LAYOUT_STREAM_MAJOR", "LAYOUT_TILED", "BUS_NONE", "SPACE_HOST", "SPACE_DEVICE", "library_path",
+    "LAYOUT_STREAM_MAJOR", "LAYOUT_TILED", "BUS_NONE", "MAX_ROUTES", "SPACE_HOST", "SPACE_DEVICE", "library_path",
     "load_library", "build_info", "plan_placement",
 ]

@@ -10,6 +10,7 @@
 
 #include <cstddef>
 #include <cstdint>
+#include <cstdlib>
 #include <string>
 
 #include "bus.cuh"
@@ -34,6 +35,9 @@ public:
 	// Page-lock / release a caller's host buffer (no-ops in the CPU test backend).
 	virtual bool host_register(void*, size_t) { return true; }
 	virtual void host_unregister(void*) {}
+	// Page-locked host memory of the engine's own (zero-filled, or null); plain heap memory in the CPU test backend.
+	virtual void* host_alloc(size_t bytes) { return std::calloc(bytes ? bytes : 1, 1); }
+	virtual void host_free(void* p) { std::free(p); }
 	// dst/src are device pointers; rows of `width` bytes.
 	virtual bool copy_2d(void* dst, size_t dst_pitch, const void* src, size_t src_pitch, size_t width, size_t rows,
 		void* stream) = 0;

@@ -13,6 +13,10 @@
 //   a bus's last run writes its row of `buses` directly, every other run a partial row in the scratch arena.
 // run_sum is the element body of every level, on the device (k_bus.cu) and in the host loop below (the Backend default,
 // which the CPU test backend runs).
+//
+// Routes (oalsfx_engine_set_routes): a stream may feed up to four buses, each through its own gain.  A member is then one
+// (stream, bus) route, its level-0 value gain(T) * x with T the frame's clock value; route_gain is the one definition of
+// gain(T), for the kernels, the host loop and the engine's start gains.  A chunk without gains (a unity plan) reads x.
 #ifndef OALSFX_BUS_CUH
 #define OALSFX_BUS_CUH
 
@@ -39,6 +43,30 @@ struct Run {
 	int32_t src, count, dst;
 };
 
+// A route's gain parameters: start gain g0, target g1, ramp length rf (frames) and ramp start t0 (frame clock).
+struct RouteGain {
+	float g0, g1;
+	int32_t rf, pad;
+	long long t0;
+};
+
+// The gain at clock value t (the header's contract): g0 before t0, g1 from t0 + rf on (or at once when rf == 0), the
+// linear ramp in between, every operation rounded on its own (no contraction: -fmad=false / -ffp-contract=off).
+OALSFX_HD float route_gain(const RouteGain& p, long long t)
+{
+	if (t < p.t0) {
+		return p.g0;
+	}
+	const long long d = t - p.t0;
+	if (p.rf == 0 || d >= p.rf) {
+		return p.g1;
+	}
+	const float diff = p.g1 - p.g0;
+	const float frac = static_cast<float>(static_cast<int32_t>(d) + 1) / static_cast<float>(p.rf);   // (d < rf <= 2^24)
+	const float step = diff * frac;
+	return p.g0 + step;
+}
+
 // One pass over frames [f0, f0 + nf) of a call of `frames` frames.  Level L's partial rows hold nf * channels floats each
 // ([frame][channel]), row r at partial[L] + r * nf * channels.
 struct Chunk {
@@ -51,6 +79,9 @@ struct Chunk {
 	int n_runs[kBusMaxLevels];
 	float* partial[kBusMaxLevels];
 	float* buses;                     // bus b, frame f, channel c at buses[(b * frames + f) * channels + c]
+	const RouteGain* gains;           // device, per member entry; null: every member's gain is 1 over the chunk (unity)
+	long long clock;                  // frame clock value of frame 0 of the call (M): frame f is at clock + f
+	bool ramping;                     // with gains: some member's gain changes inside the chunk; else each is its g1
 };
 
 struct Vec4 {
@@ -86,7 +117,8 @@ struct HostLoad {
 		}
 		const int s = k->members[run.src + i];
 		const long long f = k->f0 + j / k->channels, c = j % k->channels;
-		return k->dst[(s / kLanes) * k->ts + (s % kLanes) * k->ls + f * k->fs + c * k->cs];
+		const float x = k->dst[(s / kLanes) * k->ts + (s % kLanes) * k->ls + f * k->fs + c * k->cs];
+		return k->gains ? route_gain(k->gains[run.src + i], k->clock + f) * x : x;
 	}
 };
 

@@ -7,6 +7,7 @@
 
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <string>
 #include <vector>
 
@@ -321,6 +322,22 @@ public:
 	{
 		if (cudaHostUnregister(p) != cudaSuccess) {
 			cudaGetLastError();
+		}
+	}
+	void* host_alloc(size_t bytes) override
+	{
+		DeviceScope scope(this);
+		void* p = nullptr;
+		if (!scope.ok || !check(cudaHostAlloc(&p, bytes ? bytes : 1, cudaHostAllocDefault), "cudaHostAlloc")) {
+			return nullptr;
+		}
+		std::memset(p, 0, bytes);
+		return p;
+	}
+	void host_free(void* p) override
+	{
+		if (p) {
+			cudaFreeHost(p);
 		}
 	}
 

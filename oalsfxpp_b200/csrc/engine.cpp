@@ -167,14 +167,25 @@ struct oalsfx_engine {
 	int lane_count() const { return placed ? arena_tiles * kLanes : streams; }
 	int lane_of(int s) const { return placed ? lane_of_stream[static_cast<size_t>(s)] : s; }
 
-	// Submix buses (oalsfx_engine_route_streams / reduce_buses, bus.cuh).  The routing is kept in caller order; the plan --
-	// the members of every bus (its active streams, ascending) and the runs of every level of the summation tree -- depends
-	// on caller streams and activity only, is rebuilt on the host at the first reduce after a routing or activity change
-	// and uploaded once.  Lane moves do not touch it.
-	std::vector<int32_t> bus_of_stream;  // OALSFX_BUS_NONE (-1) or a bus index, per caller stream
-	int max_bus = 0;                     // largest bus index any stream is routed to (-1: none)
+	// Submix buses (oalsfx_engine_set_routes / route_streams / reduce_buses, bus.cuh).  The routes are kept in caller
+	// order; the plan -- the members of every bus (the routes to it of active streams, ascending stream index) and the runs
+	// of every level of the summation tree -- depends on caller streams, the (stream, bus) pairs and activity only, is
+	// rebuilt on the host at the first reduce after such a change and uploaded once.  Lane moves do not touch it.  A change
+	// of gains or ramps alone rewrites the routes' entries of the gain image, uploaded at the next reduce.
+	std::vector<int32_t> route_bus;          // stream s's routes at [s * OALSFX_MAX_ROUTES, +OALSFX_MAX_ROUTES): used ones first, then OALSFX_BUS_NONE
+	std::vector<bus::RouteGain> route_gain;  // their gain parameters
+	std::vector<int32_t> route_entry;        // their entries in the member list (-1: none: a free slot or a paused stream)
+	int max_bus = 0;                     // largest bus index any route names (-1: none)
 	bool bus_plan_dirty = true;
 	std::vector<int32_t> bus_plan;       // host image of bus_plan_dev: the member list, then every level's runs
+	int bus_entries = 0;                 // length of the member list
+	bus::RouteGain* gain_host = nullptr; // page-locked image of gain_dev: per member entry its route's gains
+	size_t gain_host_cap = 0;            // entries
+	bus::RouteGain* gain_dev = nullptr;
+	size_t gain_dev_cap = 0;             // entries
+	bool gains_dirty = false;            // gain_host changed since the last upload
+	bool gains_unity = true;             // every member's g1 is 1.0f ...
+	long long gains_ramp_end = 0;        // ... and from this clock value on every member's gain is its g1
 	int bus_levels = 0;
 	size_t bus_run_word[bus::kBusMaxLevels] = {};       // word offset of the level's runs in the plan
 	int bus_runs[bus::kBusMaxLevels] = {};
@@ -196,6 +207,10 @@ struct oalsfx_engine {
 	bool groups_dirty = true;
 	long long launches = 0;
 	int last_kernel = -1;               // id of the most recent mix kernel launched (oalsfx_engine_last_kernel)
+	// The frame clock (include/oalsfx_engine.h): frames mixed by successful mix / mix_bus / mix_buses calls, and its value
+	// at the start of the most recent one (frame f of a reduce_buses block is at clock_mix + f).
+	long long clock_total = 0;
+	long long clock_mix = 0;
 	// Host buffers the engine has page-locked in place (oalsfx_engine_pin_host, or on first sight with OALSFX_PIN_HOST=1)
 	struct PinnedHost { void* p; size_t bytes; bool automatic; };
 	std::vector<PinnedHost> pinned_host;
@@ -289,6 +304,8 @@ struct oalsfx_engine {
 		be->release(io_out);
 		be->release(bus_plan_dev);
 		be->release(bus_scratch);
+		be->release(gain_dev);
+		be->host_free(gain_host);
 		be->stream_destroy(pipe_in);
 		be->stream_destroy(pipe_run);
 		be->stream_destroy(pipe_out);
@@ -560,30 +577,49 @@ struct oalsfx_engine {
 		return nullptr;
 	}
 
-	// Members of every bus 0..max_bus in CSR order, then level by level: a bus whose list has one run left ends in that
-	// run (it writes the bus row), every other bus cuts its list into runs of 32 that write partial rows, which are the
-	// bus's list at the next level.
+	// Members of every bus 0..max_bus in CSR order (one entry per route of an active stream: its stream index; its gains at
+	// the same index of gain_host), then level by level: a bus whose list has one run left ends in that run (it writes the
+	// bus row), every other bus cuts its list into runs of 32 that write partial rows, which are the bus's list at the
+	// next level.
 	bool rebuild_bus_plan(void* stream)
 	{
 		const int nb = max_bus + 1;
+		const size_t routes = route_bus.size();
 		std::vector<int32_t> start(static_cast<size_t>(nb) + 1, 0);
-		for (int s = 0; s < streams; ++s) {
-			const int b = bus_of_stream[static_cast<size_t>(s)];
-			if (b >= 0 && active[static_cast<size_t>(lane_of(s))]) {
+		for (size_t r = 0; r < routes; ++r) {
+			const int b = route_bus[r];
+			if (b >= 0 && active[static_cast<size_t>(lane_of(static_cast<int>(r / OALSFX_MAX_ROUTES)))]) {
 				++start[static_cast<size_t>(b) + 1];
 			}
 		}
 		for (int b = 0; b < nb; ++b) {
 			start[static_cast<size_t>(b) + 1] += start[static_cast<size_t>(b)];
 		}
-		bus_plan.assign(static_cast<size_t>(start[static_cast<size_t>(nb)]), 0);
+		bus_entries = start[static_cast<size_t>(nb)];
+		if (static_cast<size_t>(bus_entries) > gain_host_cap) {
+			// (nothing reads the old image: the route and activity calls that dirty the plan wait for the caller's stream)
+			be->host_free(gain_host);
+			gain_host_cap = 0;
+			gain_host = static_cast<bus::RouteGain*>(be->host_alloc(static_cast<size_t>(bus_entries) * sizeof(bus::RouteGain)));
+			if (!gain_host) {
+				return false;
+			}
+			gain_host_cap = static_cast<size_t>(bus_entries);
+		}
+		bus_plan.assign(static_cast<size_t>(bus_entries), 0);
 		std::vector<int32_t> fill(start.begin(), start.end() - 1);
-		for (int s = 0; s < streams; ++s) {
-			const int b = bus_of_stream[static_cast<size_t>(s)];
+		for (size_t r = 0; r < routes; ++r) {
+			const int b = route_bus[r];
+			const int s = static_cast<int>(r / OALSFX_MAX_ROUTES);
+			route_entry[r] = -1;
 			if (b >= 0 && active[static_cast<size_t>(lane_of(s))]) {
-				bus_plan[static_cast<size_t>(fill[static_cast<size_t>(b)]++)] = s;
+				const int32_t entry = fill[static_cast<size_t>(b)]++;
+				bus_plan[static_cast<size_t>(entry)] = s;
+				gain_host[entry] = route_gain[r];
+				route_entry[r] = entry;
 			}
 		}
+		gains_dirty = true;
 		struct List {
 			int bus;
 			int32_t src, len;
@@ -633,13 +669,51 @@ struct oalsfx_engine {
 		return true;
 	}
 
+	// After a change of gain_host: whether every member's gain is 1 (gains_unity) from which clock value on
+	// (gains_ramp_end), and the upload of the image unless no chunk from now on needs it (a steady unity plan: the clock
+	// only grows, and the next change of gains marks the image dirty again).
+	bool upload_gains(void* stream)
+	{
+		gains_unity = true;
+		gains_ramp_end = 0;
+		for (int i = 0; i < bus_entries; ++i) {
+			const bus::RouteGain& g = gain_host[i];
+			gains_unity = gains_unity && g.g1 == 1.0F;
+			if (g.g0 != g.g1) {   // (g0 == g1: route_gain is g1 at every t, up to the sign of a zero, which no bus sum shows)
+				gains_ramp_end = std::max(gains_ramp_end, g.t0 + g.rf);
+			}
+		}
+		if (!(gains_unity && gains_ramp_end <= clock_mix) && bus_entries > 0) {
+			if (static_cast<size_t>(bus_entries) > gain_dev_cap) {
+				quiesce();   // a reduce may still read the old array
+				be->release(gain_dev);
+				device_bytes -= static_cast<long long>(gain_dev_cap * sizeof(bus::RouteGain));
+				gain_dev_cap = 0;
+				gain_dev = static_cast<bus::RouteGain*>(dev_alloc(gain_host_cap * sizeof(bus::RouteGain)));
+				if (!gain_dev) {
+					return false;
+				}
+				gain_dev_cap = gain_host_cap;
+			}
+			if (!be->upload(gain_dev, gain_host, static_cast<size_t>(bus_entries) * sizeof(bus::RouteGain), stream)) {
+				return false;
+			}
+		}
+		gains_dirty = false;
+		return true;
+	}
+
 	// oalsfx_engine_reduce_buses with checked arguments: chunks of <= kBusChunkFrames frames, one launch per level each;
-	// buses above every routed index have no members and are zeroed.
+	// buses above every routed index have no members and are zeroed.  A chunk whose members all have gain 1 over its frames
+	// runs the plain sum; any other reads the gains, steady (each member at its g1) or ramping.
 	int reduce_buses(int frames, const float* dst, int layout, int n_buses, float* buses, void* stream)
 	{
 		note_stream(stream);
 		if (bus_plan_dirty && !rebuild_bus_plan(stream)) {
 			return fail(OALSFX_ERR_DEVICE, "Bus plan upload failed: " + be->error());
+		}
+		if (gains_dirty && !upload_gains(stream)) {
+			return fail(OALSFX_ERR_DEVICE, "Route gain upload failed: " + be->error());
 		}
 		const int chunk = std::min(frames, bus::kBusChunkFrames);
 		const size_t need = static_cast<size_t>(bus_partial_rows) * static_cast<size_t>(chunk) * static_cast<size_t>(channels);
@@ -666,6 +740,7 @@ struct oalsfx_engine {
 		k.members = bus_plan_dev;
 		k.levels = bus_levels;
 		k.buses = buses;
+		k.clock = clock_mix;
 		for (int level = 0; level < bus_levels; ++level) {
 			k.runs[level] = reinterpret_cast<const bus::Run*>(bus_plan_dev + bus_run_word[level]);
 			k.n_runs[level] = bus_runs[level];
@@ -673,6 +748,8 @@ struct oalsfx_engine {
 		for (int f0 = 0; f0 < frames; f0 += bus::kBusChunkFrames) {
 			k.f0 = f0;
 			k.nf = std::min(frames - f0, bus::kBusChunkFrames);
+			k.ramping = clock_mix + f0 < gains_ramp_end;
+			k.gains = gains_unity && !k.ramping ? nullptr : gain_dev;
 			for (int level = 0; level < bus_levels; ++level) {
 				k.partial[level] = bus_scratch ? bus_scratch + bus_partial_row[level] * k.nf * channels : nullptr;
 			}
@@ -2013,7 +2090,13 @@ int oalsfx_engine_create(const oalsfx_engine_desc* desc, oalsfx_engine** out)
 	e->send_class.assign(static_cast<size_t>(e->streams), e->send_class_for(unit, aux));
 	e->pending.assign(static_cast<size_t>(e->streams), 0);
 	e->active.assign(static_cast<size_t>(e->streams), 1);
-	e->bus_of_stream.assign(static_cast<size_t>(e->streams), 0);
+	// every stream routed to bus 0 at gain 1
+	e->route_bus.assign(static_cast<size_t>(e->streams) * OALSFX_MAX_ROUTES, OALSFX_BUS_NONE);
+	e->route_gain.assign(e->route_bus.size(), bus::RouteGain{1.0F, 1.0F, 0, 0, 0});
+	e->route_entry.assign(e->route_bus.size(), -1);
+	for (int s = 0; s < e->streams; ++s) {
+		e->route_bus[static_cast<size_t>(s) * OALSFX_MAX_ROUTES] = 0;
+	}
 	*out = e;
 	return OALSFX_OK;
 }
@@ -2174,34 +2257,98 @@ int oalsfx_engine_reset_streams(oalsfx_engine* e, int first_stream, int n_stream
 	return OALSFX_OK;
 }
 
-int oalsfx_engine_route_streams(oalsfx_engine* e, int first_stream, int n_streams, const int32_t* bus)
+int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream, const int32_t* bus,
+	const float* gain, int ramp_frames)
 {
 	if (!e) {
 		return OALSFX_ERR_ARGUMENT;
 	}
+	const int R = routes_per_stream;
 	if (first_stream < 0 || n_streams < 1 || first_stream + n_streams > e->streams || !bus) {
 		return e->fail(OALSFX_ERR_ARGUMENT, "Bad stream range or null bus list.");
 	}
+	if (R < 1 || R > OALSFX_MAX_ROUTES) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "routes_per_stream must be 1..OALSFX_MAX_ROUTES.");
+	}
+	if (ramp_frames < 0 || ramp_frames > (1 << 24)) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "ramp_frames must be 0..2^24.");
+	}
 	for (int i = 0; i < n_streams; ++i) {
-		if (bus[i] < OALSFX_BUS_NONE) {
-			return e->fail(OALSFX_ERR_ARGUMENT, "Bus index below OALSFX_BUS_NONE.");
+		for (int r = 0; r < R; ++r) {
+			const int32_t b = bus[i * R + r];
+			if (b < OALSFX_BUS_NONE) {
+				return e->fail(OALSFX_ERR_ARGUMENT, "Bus index below OALSFX_BUS_NONE.");
+			}
+			for (int q = 0; q < r && b != OALSFX_BUS_NONE; ++q) {
+				if (bus[i * R + q] == b) {
+					return e->fail(OALSFX_ERR_ARGUMENT, "A stream names the same bus twice.");
+				}
+			}
+			if (gain && b != OALSFX_BUS_NONE && !std::isfinite(gain[i * R + r])) {
+				return e->fail(OALSFX_ERR_ARGUMENT, "Route gains must be finite.");
+			}
 		}
 	}
 	e->quiesce();
-	bool changed = false;
+	const long long t0 = e->clock_total;
+	bool pairs_changed = false;
 	for (int i = 0; i < n_streams; ++i) {
-		int32_t& cur = e->bus_of_stream[static_cast<size_t>(first_stream + i)];
-		changed = changed || cur != bus[i];
-		cur = bus[i];
+		int32_t* cur = e->route_bus.data() + static_cast<size_t>(first_stream + i) * OALSFX_MAX_ROUTES;
+		bus::RouteGain* cur_gain = e->route_gain.data() + (cur - e->route_bus.data());
+		int32_t new_bus[OALSFX_MAX_ROUTES];
+		bus::RouteGain new_gain[OALSFX_MAX_ROUTES];
+		int old_slot[OALSFX_MAX_ROUTES];
+		int n = 0;
+		bool same = true;   // the same (stream, bus) pairs: every route keeps its slot and member entry, only its gains change
+		for (int r = 0; r < R; ++r) {
+			const int32_t b = bus[i * R + r];
+			if (b == OALSFX_BUS_NONE) {
+				continue;
+			}
+			int k = 0;
+			while (k < OALSFX_MAX_ROUTES && cur[k] != b) {
+				++k;
+			}
+			// the start gain: the route's gain at the last mixed frame, or 0 for a new route; without a ramp the new gain holds
+			// at once, also for a block mixed before the call
+			const float g1 = gain ? gain[i * R + r] : 1.0F;
+			const float g0 = ramp_frames == 0 ? g1 : k < OALSFX_MAX_ROUTES ? bus::route_gain(cur_gain[k], t0 - 1) : 0.0F;
+			same = same && k < OALSFX_MAX_ROUTES;
+			old_slot[n] = k;
+			new_bus[n] = b;
+			new_gain[n] = bus::RouteGain{g0, g1, ramp_frames, 0, t0};
+			++n;
+		}
+		same = same && (n == OALSFX_MAX_ROUTES || cur[n] == OALSFX_BUS_NONE);   // (used slots come first)
+		for (int r = 0; r < n && same; ++r) {
+			const size_t k = static_cast<size_t>(cur - e->route_bus.data() + old_slot[r]);
+			e->route_gain[k] = new_gain[r];
+			if (e->route_entry[k] >= 0) {
+				e->gain_host[e->route_entry[k]] = new_gain[r];
+				e->gains_dirty = true;
+			}
+		}
+		if (!same) {
+			for (int k = 0; k < OALSFX_MAX_ROUTES; ++k) {
+				cur[k] = k < n ? new_bus[k] : OALSFX_BUS_NONE;
+				cur_gain[k] = k < n ? new_gain[k] : bus::RouteGain{};
+			}
+			pairs_changed = true;
+		}
 	}
-	if (changed) {
-		e->max_bus = *std::max_element(e->bus_of_stream.begin(), e->bus_of_stream.end());
+	if (pairs_changed) {
+		e->max_bus = *std::max_element(e->route_bus.begin(), e->route_bus.end());
 		e->bus_plan_dirty = true;
 	}
 	return OALSFX_OK;
 }
 
-int oalsfx_engine_mix(oalsfx_engine* e, int frames, const float* src, float* dst, int layout, int space, void* cuda_stream)
+int oalsfx_engine_route_streams(oalsfx_engine* e, int first_stream, int n_streams, const int32_t* bus)
+{
+	return oalsfx_engine_set_routes(e, first_stream, n_streams, 1, bus, nullptr, 0);
+}
+
+static int mix_blocks(oalsfx_engine* e, int frames, const float* src, float* dst, int layout, int space, void* cuda_stream)
 {
 	if (!e) {
 		return OALSFX_ERR_ARGUMENT;
@@ -2384,6 +2531,18 @@ int oalsfx_engine_mix(oalsfx_engine* e, int frames, const float* src, float* dst
 		}
 	}
 	return OALSFX_OK;
+}
+
+// Every mix entry point (mix, mix_bus, mix_buses) comes through here: a successful call of `frames` frames advances the
+// frame clock; a refused or failed one leaves it.
+int oalsfx_engine_mix(oalsfx_engine* e, int frames, const float* src, float* dst, int layout, int space, void* cuda_stream)
+{
+	const int rc = mix_blocks(e, frames, src, dst, layout, space, cuda_stream);
+	if (rc == OALSFX_OK && frames > 0) {
+		e->clock_mix = e->clock_total;
+		e->clock_total += frames;
+	}
+	return rc;
 }
 
 int oalsfx_engine_pin_host(oalsfx_engine* e, void* buffer, size_t bytes)

@@ -16,6 +16,7 @@ from .props import EffectProps, EffectType, channel_count
 LAYOUT_STREAM_MAJOR = 0
 LAYOUT_TILED = 1
 BUS_NONE = -1
+MAX_ROUTES = 4
 SPACE_HOST = 0
 SPACE_DEVICE = 1
 
@@ -68,6 +69,8 @@ def bind(lib):
     lib.oalsfx_engine_reduce_bus.restype = i32
     lib.oalsfx_engine_route_streams.argtypes = [vp, i32, i32, vp]
     lib.oalsfx_engine_route_streams.restype = i32
+    lib.oalsfx_engine_set_routes.argtypes = [vp, i32, i32, i32, vp, vp, i32]
+    lib.oalsfx_engine_set_routes.restype = i32
     lib.oalsfx_engine_reduce_buses.argtypes = [vp, i32, vp, i32, i32, vp, vp]
     lib.oalsfx_engine_reduce_buses.restype = i32
     lib.oalsfx_engine_mix_buses.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp]
@@ -116,7 +119,7 @@ def bind(lib):
 EXPORTED_SYMBOLS = (
     "oalsfx_engine_create", "oalsfx_engine_destroy", "oalsfx_engine_set_effect",
     "oalsfx_engine_set_sends", "oalsfx_engine_set_active", "oalsfx_engine_reset_streams", "oalsfx_engine_mix", "oalsfx_engine_mix_bus", "oalsfx_engine_reduce_bus",
-    "oalsfx_engine_route_streams", "oalsfx_engine_reduce_buses", "oalsfx_engine_mix_buses",
+    "oalsfx_engine_route_streams", "oalsfx_engine_set_routes", "oalsfx_engine_reduce_buses", "oalsfx_engine_mix_buses",
     "oalsfx_engine_pin_host", "oalsfx_engine_unpin_host",
     "oalsfx_engine_debug_state", "oalsfx_debug_waveshaper", "oalsfx_plan_placement", "oalsfx_engine_launch_count", "oalsfx_engine_last_kernel", "oalsfx_engine_device_bytes",
     "oalsfx_last_error", "oalsfx_build_info", "oalsfx_effect_defaults", "oalsfx_effect_normalize",
@@ -285,6 +288,21 @@ class Engine:
         """Route streams first_stream, first_stream + 1, ... to the buses in `bus` (ints; BUS_NONE = -1: no bus)."""
         bus = np.ascontiguousarray(bus, dtype=np.int32).ravel()
         self._check(self.lib.oalsfx_engine_route_streams(self._h, int(first_stream), int(bus.size), bus.ctypes.data))
+
+    def set_routes(self, bus, gain=None, first_stream=0, ramp_frames=0):
+        """Routes of streams first_stream, first_stream + 1, ...: bus[i] (up to MAX_ROUTES bus indices, BUS_NONE for none)
+        with gains gain[i] (default 1.0), each gain ramped from the route's current one over ramp_frames frames (a new
+        route from 0).  `bus` and `gain` are [n][R] arrays; a 1-D array means one route per stream."""
+        bus = np.asarray(bus, dtype=np.int32)
+        if bus.ndim == 1:
+            bus = bus[:, None]
+        bus = np.ascontiguousarray(bus)
+        n, R = bus.shape
+        g = None
+        if gain is not None:
+            g = np.ascontiguousarray(np.asarray(gain, dtype=np.float32).reshape(bus.shape))
+        self._check(self.lib.oalsfx_engine_set_routes(self._h, int(first_stream), int(n), int(R), bus.ctypes.data,
+                                                      None if g is None else g.ctypes.data, int(ramp_frames)))
 
     def _bus_count(self, frames, buses, n_buses):
         if n_buses is not None:
