@@ -192,6 +192,43 @@ int oalsfx_engine_route_streams(oalsfx_engine* e, int first_stream, int n_stream
 enum { OALSFX_MAX_ROUTES = 4 };
 int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream,
 	const int32_t* bus, const float* gain, int ramp_frames);
+/* Bus format and pans.  A host with mono voices and a stereo or 5.1 output, or one listener bus per player in split screen,
+ * pans each voice into each bus with gains of its own, in the buses' deterministic order.
+ * oalsfx_engine_set_bus_format: every submix bus gets the channel format `channel_format` (an oalsfxpp::ChannelFormat value,
+ * as in oalsfx_engine_desc) and Cb = its channel count (1..8); the default is the engine's own format (Cb = C).  From then
+ * on reduce_buses / mix_buses write buses[(b * frames + f) * Cb + j], n_buses * frames * Cb floats, in both layouts; the
+ * all-streams bus of reduce_bus / mix_bus keeps the engine's format.  OALSFX_ERR_FORMAT for an invalid format;
+ * OALSFX_ERR_ARGUMENT, with nothing changed, for a change of Cb while any route is a pan route (its matrix is sized for the
+ * old Cb); setting the current format again always succeeds.  Waits for the stream the caller last passed in, as
+ * set_routes does.  The bus format is configuration: reset_streams, set_placement and restore keep it, snapshots do not
+ * hold it.
+ * oalsfx_engine_set_route_pans: as set_routes -- the same `bus` array, the same checks, nothing changed by a refused call,
+ * every route of a listed stream that the call does not name removed -- but each named route r of stream first_stream + i
+ * gets a Cb x C matrix instead of a gain: pan[((i * R + r) * Cb + j) * C + k] is the weight of stream channel k in bus
+ * channel j.  OALSFX_ERR_ARGUMENT also for a null `pan` or a coefficient of a named route that is not finite.
+ *   - Scalar routes (route_streams, set_routes, the default routing) feed bus channel j < min(C, Cb) with g(T) * x_j and
+ *     bus channels j >= C with nothing.  With Cb == C this is the plain routing above, with the same kernels and bits.
+ *     With Cb != C the mapping is by index: a mono engine routed by default feeds only the left channel of a stereo bus,
+ *     and a stereo voice routed to a mono bus feeds it its left channel.  Pan the voice to mix its channels.
+ *   - A pan route's value in bus channel j is, in fp32 with one rounding per operation and no contraction,
+ *     p = c_j0(T) * x_0, then p = p + c_jk(T) * x_k for k = 1..C-1.  Every coefficient takes part (0 * Inf is NaN, as for a
+ *     route of gain 0).  Each coefficient ramps as a gain does: c_jk(T) is the gain expression above with g0_jk, g1_jk and
+ *     the route's Rf and T0.  set_route_pans sets T0 = the clock now, Rf = ramp_frames, g1 = the new matrix, and g0 = each
+ *     coefficient's value at T0 - 1 when the stream already had a route to that bus, else 0.0f (a scalar route's matrix is
+ *     its gain g(T0 - 1) where j == k and 0.0f elsewhere); with ramp_frames == 0, g0 = g1 and the matrix applies at once,
+ *     also to a block mixed before the call.
+ *   - set_routes / route_streams on a pan route: with ramp_frames == 0 it becomes a scalar route at once; with a ramp it
+ *     stays a pan route whose target is the gain on the index diagonal (j == k) and 0.0f elsewhere, so that the other
+ *     coefficients ramp out, and a later call without a ramp makes it scalar (the crossfade idiom above).
+ *   - The members and their order are those above; a member's value is now per (frame, bus channel).  So the buses stay
+ *     bit-identical across layouts, placements, repeated reduces and the cut of a call into blocks.  With Cb == C an
+ *     identity matrix times g gives the bits of set_routes(g) for a finite block (the extra terms are +-0.0f, and a run sum
+ *     starting from +0.0f never becomes -0.0f); with C == Cb == 1 a pan route is bit-identical to a scalar route.
+ *   - A set_route_pans that keeps every (stream, bus) pair costs one upload of the coefficients at the next reduce, as a
+ *     gain change does; a change of the pairs rebuilds the plan.  Pan coefficients on the device count in device_bytes. */
+int oalsfx_engine_set_bus_format(oalsfx_engine* e, int channel_format);
+int oalsfx_engine_set_route_pans(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream,
+	const int32_t* bus, const float* pan, int ramp_frames);
 int oalsfx_engine_reduce_buses(oalsfx_engine* e, int frames, const float* dst, int layout,
 	int n_buses, float* buses, void* cuda_stream);
 int oalsfx_engine_mix_buses(oalsfx_engine* e, int frames, const float* src, float* dst, int layout,

@@ -171,9 +171,13 @@ struct oalsfx_engine {
 	// order; the plan -- the members of every bus (the routes to it of active streams, ascending stream index) and the runs
 	// of every level of the summation tree -- depends on caller streams, the (stream, bus) pairs and activity only, is
 	// rebuilt on the host at the first reduce after such a change and uploaded once.  Lane moves do not touch it.  A change
-	// of gains or ramps alone rewrites the routes' entries of the gain image, uploaded at the next reduce.
+	// of gains or ramps alone rewrites the routes' entries of the gain image, uploaded at the next reduce.  Pan routes
+	// (oalsfx_engine_set_route_pans) keep their matrices beside the gains, and the plan's entries of them in the pan image.
 	std::vector<int32_t> route_bus;          // stream s's routes at [s * OALSFX_MAX_ROUTES, +OALSFX_MAX_ROUTES): used ones first, then OALSFX_BUS_NONE
-	std::vector<bus::RouteGain> route_gain;  // their gain parameters
+	std::vector<bus::RouteGain> route_gain;  // their gain parameters (pan != 0: a pan route; rf and t0 are its ramp's)
+	std::vector<std::vector<float>> route_pan; // a pan route's g0 and g1 matrices ([bus channel][channel] each); empty: scalar
+	long long pan_routes = 0;                // routes with a matrix (0: set_routes calls leave route_pan untouched)
+	int bus_channels = 0;                    // channel count Cb of the submix buses (oalsfx_engine_set_bus_format)
 	std::vector<int32_t> route_entry;        // their entries in the member list (-1: none: a free slot or a paused stream)
 	int max_bus = 0;                     // largest bus index any route names (-1: none)
 	bool bus_plan_dirty = true;
@@ -186,6 +190,11 @@ struct oalsfx_engine {
 	bool gains_dirty = false;            // gain_host changed since the last upload
 	bool gains_unity = true;             // every member's g1 is 1.0f ...
 	long long gains_ramp_end = 0;        // ... and from this clock value on every member's gain is its g1
+	bool gains_pan = false;              // some member is a pan route: level 0 runs the pan kernels (as with bus_channels != channels)
+	float* pan_host = nullptr;           // page-locked image of pan_dev: per member entry bus::pan_stride floats (used by pan routes)
+	size_t pan_host_cap = 0;             // floats; >= bus_entries * pan_stride whenever a member entry is a pan route
+	float* pan_dev = nullptr;
+	size_t pan_dev_cap = 0;              // floats
 	int bus_levels = 0;
 	size_t bus_run_word[bus::kBusMaxLevels] = {};       // word offset of the level's runs in the plan
 	int bus_runs[bus::kBusMaxLevels] = {};
@@ -306,6 +315,8 @@ struct oalsfx_engine {
 		be->release(bus_scratch);
 		be->release(gain_dev);
 		be->host_free(gain_host);
+		be->release(pan_dev);
+		be->host_free(pan_host);
 		be->stream_destroy(pipe_in);
 		be->stream_destroy(pipe_run);
 		be->stream_destroy(pipe_out);
@@ -606,6 +617,20 @@ struct oalsfx_engine {
 			}
 			gain_host_cap = static_cast<size_t>(bus_entries);
 		}
+		const size_t stride = static_cast<size_t>(bus::pan_stride(bus_channels, channels));
+		bool any_pan = false;
+		for (size_t r = 0; r < routes && !any_pan; ++r) {
+			any_pan = route_bus[r] >= 0 && !route_pan[r].empty();
+		}
+		if (any_pan && static_cast<size_t>(bus_entries) * stride > pan_host_cap) {
+			be->host_free(pan_host);
+			pan_host_cap = 0;
+			pan_host = static_cast<float*>(be->host_alloc(static_cast<size_t>(bus_entries) * stride * sizeof(float)));
+			if (!pan_host) {
+				return false;
+			}
+			pan_host_cap = static_cast<size_t>(bus_entries) * stride;
+		}
 		bus_plan.assign(static_cast<size_t>(bus_entries), 0);
 		std::vector<int32_t> fill(start.begin(), start.end() - 1);
 		for (size_t r = 0; r < routes; ++r) {
@@ -616,6 +641,9 @@ struct oalsfx_engine {
 				const int32_t entry = fill[static_cast<size_t>(b)]++;
 				bus_plan[static_cast<size_t>(entry)] = s;
 				gain_host[entry] = route_gain[r];
+				if (!route_pan[r].empty()) {
+					std::memcpy(pan_host + static_cast<size_t>(entry) * stride, route_pan[r].data(), stride * sizeof(float));
+				}
 				route_entry[r] = entry;
 			}
 		}
@@ -669,21 +697,50 @@ struct oalsfx_engine {
 		return true;
 	}
 
-	// After a change of gain_host: whether every member's gain is 1 (gains_unity) from which clock value on
-	// (gains_ramp_end), and the upload of the image unless no chunk from now on needs it (a steady unity plan: the clock
-	// only grows, and the next change of gains marks the image dirty again).
+	// Whether level 0 runs the pan kernels: some member is a pan route, or the buses have a channel count of their own.
+	bool pan_plan() const { return gains_pan || bus_channels != channels; }
+
+	// After a change of gain_host (or of the bus format): whether every member's gain is 1 (gains_unity) from which clock
+	// value on (gains_ramp_end; a pan route's coefficients count as its gains), whether some member is a pan route
+	// (gains_pan), and the upload of the images unless no chunk from now on needs them (a steady unity plan of scalar routes
+	// into buses of the engine's format: the clock only grows, and the next change of gains marks the image dirty again).
 	bool upload_gains(void* stream)
 	{
 		gains_unity = true;
 		gains_ramp_end = 0;
+		gains_pan = false;
+		const int stride = bus::pan_stride(bus_channels, channels);
 		for (int i = 0; i < bus_entries; ++i) {
 			const bus::RouteGain& g = gain_host[i];
-			gains_unity = gains_unity && g.g1 == 1.0F;
-			if (g.g0 != g.g1) {   // (g0 == g1: route_gain is g1 at every t, up to the sign of a zero, which no bus sum shows)
+			bool ramps = g.g0 != g.g1;   // (g0 == g1: route_gain is g1 at every t, up to the sign of a zero, which no bus sum shows)
+			if (g.pan) {
+				const float* m = pan_host + static_cast<size_t>(i) * static_cast<size_t>(stride);
+				ramps = !std::equal(m, m + stride / 2, m + stride / 2);
+				gains_pan = true;
+			}
+			gains_unity = gains_unity && g.g1 == 1.0F && !g.pan;
+			if (ramps) {
 				gains_ramp_end = std::max(gains_ramp_end, g.t0 + g.rf);
 			}
 		}
-		if (!(gains_unity && gains_ramp_end <= clock_mix) && bus_entries > 0) {
+		if (gains_pan) {
+			const size_t need = static_cast<size_t>(bus_entries) * static_cast<size_t>(stride);
+			if (need > pan_dev_cap) {
+				quiesce();   // a reduce may still read the old array
+				be->release(pan_dev);
+				device_bytes -= static_cast<long long>(pan_dev_cap * sizeof(float));
+				pan_dev_cap = 0;
+				pan_dev = static_cast<float*>(dev_alloc(need * sizeof(float)));
+				if (!pan_dev) {
+					return false;
+				}
+				pan_dev_cap = need;
+			}
+			if (!be->upload(pan_dev, pan_host, need * sizeof(float), stream)) {
+				return false;
+			}
+		}
+		if ((!(gains_unity && gains_ramp_end <= clock_mix) || pan_plan()) && bus_entries > 0) {
 			if (static_cast<size_t>(bus_entries) > gain_dev_cap) {
 				quiesce();   // a reduce may still read the old array
 				be->release(gain_dev);
@@ -716,7 +773,7 @@ struct oalsfx_engine {
 			return fail(OALSFX_ERR_DEVICE, "Route gain upload failed: " + be->error());
 		}
 		const int chunk = std::min(frames, bus::kBusChunkFrames);
-		const size_t need = static_cast<size_t>(bus_partial_rows) * static_cast<size_t>(chunk) * static_cast<size_t>(channels);
+		const size_t need = static_cast<size_t>(bus_partial_rows) * static_cast<size_t>(chunk) * static_cast<size_t>(bus_channels);
 		if (need > bus_scratch_cap) {
 			quiesce();
 			be->release(bus_scratch);
@@ -737,6 +794,9 @@ struct oalsfx_engine {
 		k.cs = layout == OALSFX_LAYOUT_TILED ? kLanes : 1;
 		k.frames = frames;
 		k.channels = channels;
+		k.bus_channels = bus_channels;
+		k.pan_plan = pan_plan();
+		k.pan = pan_dev;
 		k.members = bus_plan_dev;
 		k.levels = bus_levels;
 		k.buses = buses;
@@ -749,16 +809,16 @@ struct oalsfx_engine {
 			k.f0 = f0;
 			k.nf = std::min(frames - f0, bus::kBusChunkFrames);
 			k.ramping = clock_mix + f0 < gains_ramp_end;
-			k.gains = gains_unity && !k.ramping ? nullptr : gain_dev;
+			k.gains = gains_unity && !k.ramping && !k.pan_plan ? nullptr : gain_dev;
 			for (int level = 0; level < bus_levels; ++level) {
-				k.partial[level] = bus_scratch ? bus_scratch + bus_partial_row[level] * k.nf * channels : nullptr;
+				k.partial[level] = bus_scratch ? bus_scratch + bus_partial_row[level] * k.nf * bus_channels : nullptr;
 			}
 			launches += bus_levels;
 			if (!be->reduce_buses(k, stream)) {
 				return fail(OALSFX_ERR_DEVICE, be->error());
 			}
 		}
-		const long long per_bus = static_cast<long long>(frames) * channels;
+		const long long per_bus = static_cast<long long>(frames) * bus_channels;
 		if (n_buses > max_bus + 1 && !be->zero(buses + (max_bus + 1) * per_bus,
 				static_cast<size_t>(n_buses - max_bus - 1) * static_cast<size_t>(per_bus) * sizeof(float), stream)) {
 			return fail(OALSFX_ERR_DEVICE, be->error());
@@ -2090,9 +2150,11 @@ int oalsfx_engine_create(const oalsfx_engine_desc* desc, oalsfx_engine** out)
 	e->send_class.assign(static_cast<size_t>(e->streams), e->send_class_for(unit, aux));
 	e->pending.assign(static_cast<size_t>(e->streams), 0);
 	e->active.assign(static_cast<size_t>(e->streams), 1);
-	// every stream routed to bus 0 at gain 1
+	// every stream routed to bus 0 at gain 1, buses in the engine's format
 	e->route_bus.assign(static_cast<size_t>(e->streams) * OALSFX_MAX_ROUTES, OALSFX_BUS_NONE);
 	e->route_gain.assign(e->route_bus.size(), bus::RouteGain{1.0F, 1.0F, 0, 0, 0});
+	e->route_pan.assign(e->route_bus.size(), std::vector<float>());
+	e->bus_channels = e->channels;
 	e->route_entry.assign(e->route_bus.size(), -1);
 	for (int s = 0; s < e->streams; ++s) {
 		e->route_bus[static_cast<size_t>(s) * OALSFX_MAX_ROUTES] = 0;
@@ -2257,13 +2319,52 @@ int oalsfx_engine_reset_streams(oalsfx_engine* e, int first_stream, int n_stream
 	return OALSFX_OK;
 }
 
-int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream, const int32_t* bus,
-	const float* gain, int ramp_frames)
+// A pan route's matrices (set_routes_impl): target m1 = `target` (a Cb x C matrix), or gain g1 on the index diagonal when
+// `target` is null; start m0 = m1 without a ramp, else the old route's coefficients at t0 - 1 (`old_pan`, or a scalar route's
+// gain on the diagonal, `old`), or 0 for a new route.
+static void pan_route_start(std::vector<float>& out, const float* target, float g1, int C, int Cb, int ramp_frames,
+	const std::vector<float>* old_pan, const bus::RouteGain* old, long long t0)
 {
-	if (!e) {
-		return OALSFX_ERR_ARGUMENT;
+	const int cm = Cb * C;
+	out.assign(static_cast<size_t>(2 * cm), 0.0F);
+	float* m0 = out.data();
+	float* m1 = m0 + cm;
+	if (target) {
+		std::copy_n(target, cm, m1);
+	} else {
+		for (int j = 0; j < std::min(C, Cb); ++j) {
+			m1[j * C + j] = g1;
+		}
 	}
+	if (ramp_frames == 0) {
+		std::copy_n(m1, cm, m0);
+	} else if (old_pan) {
+		const float pos = bus::ramp_pos(old->rf, old->t0, t0 - 1);
+		for (int q = 0; q < cm; ++q) {
+			m0[q] = bus::ramp_apply((*old_pan)[static_cast<size_t>(q)], (*old_pan)[static_cast<size_t>(cm + q)], pos);
+		}
+	} else if (old) {
+		const float g = bus::route_gain(*old, t0 - 1);
+		for (int j = 0; j < std::min(C, Cb); ++j) {
+			m0[j * C + j] = g;
+		}
+	}
+}
+
+extern "C++" {
+template <bool kPans>
+static int replace_routes(oalsfx_engine* e, int first_stream, int n_streams, int R, const int32_t* bus, const float* gain,
+	const float* pan, int ramp_frames);
+}
+
+// oalsfx_engine_set_routes (gain: per route, or NULL: 1.0f) and oalsfx_engine_set_route_pans (pan: per route a Cb x C
+// matrix): one body, so that both check, replace and ramp routes alike.  A route becomes a pan route through set_route_pans,
+// and stays one under set_routes with a ramp, which then ramps it to its gain on the index diagonal.
+static int set_routes_impl(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream, const int32_t* bus,
+	const float* gain, const float* pan, int ramp_frames)
+{
 	const int R = routes_per_stream;
+	const int C = e->channels, Cb = e->bus_channels, cm = Cb * C;
 	if (first_stream < 0 || n_streams < 1 || first_stream + n_streams > e->streams || !bus) {
 		return e->fail(OALSFX_ERR_ARGUMENT, "Bad stream range or null bus list.");
 	}
@@ -2287,14 +2388,39 @@ int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, 
 			if (gain && b != OALSFX_BUS_NONE && !std::isfinite(gain[i * R + r])) {
 				return e->fail(OALSFX_ERR_ARGUMENT, "Route gains must be finite.");
 			}
+			const float* m = pan ? pan + static_cast<size_t>(i * R + r) * static_cast<size_t>(cm) : nullptr;
+			if (m && b != OALSFX_BUS_NONE && !std::all_of(m, m + cm, [](float v) { return std::isfinite(v); })) {
+				return e->fail(OALSFX_ERR_ARGUMENT, "Pan coefficients must be finite.");
+			}
 		}
 	}
 	e->quiesce();
+	// without a pan route before or after the call, the loop leaves the matrices alone: set_routes keeps its cost
+	return pan || e->pan_routes > 0 ? replace_routes<true>(e, first_stream, n_streams, R, bus, gain, pan, ramp_frames) :
+		replace_routes<false>(e, first_stream, n_streams, R, bus, gain, nullptr, ramp_frames);
+}
+
+extern "C++" {
+// The routes of streams [first_stream, first_stream + n_streams) after set_routes_impl's checks.  kPans: some route has a
+// matrix, before or after the call.
+template <bool kPans>
+static int replace_routes(oalsfx_engine* e, int first_stream, int n_streams, int R, const int32_t* bus, const float* gain,
+	const float* pan, int ramp_frames)
+{
+	const int C = e->channels, Cb = e->bus_channels, cm = Cb * C;
 	const long long t0 = e->clock_total;
+	const size_t stride = static_cast<size_t>(2 * cm);
+	constexpr bool pans = kPans;
+	auto put_pan = [e](size_t slot, std::vector<float>& m) {   // slot's matrices become m's (m gets the old ones)
+		e->pan_routes += static_cast<long long>(!m.empty()) - static_cast<long long>(!e->route_pan[slot].empty());
+		e->route_pan[slot].swap(m);
+	};
 	bool pairs_changed = false;
+	std::vector<float> new_pan[OALSFX_MAX_ROUTES];   // (reused from stream to stream: swapped with the routes' matrices)
 	for (int i = 0; i < n_streams; ++i) {
-		int32_t* cur = e->route_bus.data() + static_cast<size_t>(first_stream + i) * OALSFX_MAX_ROUTES;
-		bus::RouteGain* cur_gain = e->route_gain.data() + (cur - e->route_bus.data());
+		const size_t base = static_cast<size_t>(first_stream + i) * OALSFX_MAX_ROUTES;
+		int32_t* cur = e->route_bus.data() + base;
+		bus::RouteGain* cur_gain = e->route_gain.data() + base;
 		int32_t new_bus[OALSFX_MAX_ROUTES];
 		bus::RouteGain new_gain[OALSFX_MAX_ROUTES];
 		int old_slot[OALSFX_MAX_ROUTES];
@@ -2309,29 +2435,59 @@ int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, 
 			while (k < OALSFX_MAX_ROUTES && cur[k] != b) {
 				++k;
 			}
+			const bool had = k < OALSFX_MAX_ROUTES;
+			const std::vector<float>* old_pan = pans && had && !e->route_pan[base + static_cast<size_t>(k)].empty() ?
+				&e->route_pan[base + static_cast<size_t>(k)] : nullptr;
 			// the start gain: the route's gain at the last mixed frame, or 0 for a new route; without a ramp the new gain holds
 			// at once, also for a block mixed before the call
 			const float g1 = gain ? gain[i * R + r] : 1.0F;
-			const float g0 = ramp_frames == 0 ? g1 : k < OALSFX_MAX_ROUTES ? bus::route_gain(cur_gain[k], t0 - 1) : 0.0F;
-			same = same && k < OALSFX_MAX_ROUTES;
+			if (!pans || (!pan && !(old_pan && ramp_frames > 0))) {
+				if (pans) {
+					new_pan[n].clear();
+				}
+				const float g0 = ramp_frames == 0 ? g1 : had ? bus::route_gain(cur_gain[k], t0 - 1) : 0.0F;
+				new_gain[n] = bus::RouteGain{g0, g1, ramp_frames, 0, t0};
+			} else {
+				pan_route_start(new_pan[n], pan ? pan + static_cast<size_t>(i * R + r) * static_cast<size_t>(cm) : nullptr, g1, C, Cb,
+					ramp_frames, old_pan, had ? &cur_gain[k] : nullptr, t0);
+				new_gain[n] = bus::RouteGain{0.0F, 0.0F, ramp_frames, 1, t0};
+			}
+			same = same && had;
 			old_slot[n] = k;
 			new_bus[n] = b;
-			new_gain[n] = bus::RouteGain{g0, g1, ramp_frames, 0, t0};
 			++n;
 		}
 		same = same && (n == OALSFX_MAX_ROUTES || cur[n] == OALSFX_BUS_NONE);   // (used slots come first)
 		for (int r = 0; r < n && same; ++r) {
-			const size_t k = static_cast<size_t>(cur - e->route_bus.data() + old_slot[r]);
+			const size_t k = base + static_cast<size_t>(old_slot[r]);
 			e->route_gain[k] = new_gain[r];
-			if (e->route_entry[k] >= 0) {
-				e->gain_host[e->route_entry[k]] = new_gain[r];
-				e->gains_dirty = true;
+			if (pans) {
+				put_pan(k, new_pan[r]);
+			}
+			const int entry = e->route_entry[k];
+			if (entry < 0) {
+				continue;
+			}
+			e->gain_host[entry] = new_gain[r];
+			e->gains_dirty = true;
+			if (pans && !e->route_pan[k].empty()) {
+				if (static_cast<size_t>(e->bus_entries) * stride > e->pan_host_cap) {
+					e->bus_plan_dirty = true;   // the plan's first pan route: the rebuild sizes the pan image for every entry
+				} else {
+					std::copy(e->route_pan[k].begin(), e->route_pan[k].end(), e->pan_host + static_cast<size_t>(entry) * stride);
+				}
 			}
 		}
 		if (!same) {
 			for (int k = 0; k < OALSFX_MAX_ROUTES; ++k) {
 				cur[k] = k < n ? new_bus[k] : OALSFX_BUS_NONE;
 				cur_gain[k] = k < n ? new_gain[k] : bus::RouteGain{};
+				if (pans) {
+					if (k >= n) {
+						new_pan[k].clear();   // (the slot has no route)
+					}
+					put_pan(base + static_cast<size_t>(k), new_pan[k]);
+				}
 			}
 			pairs_changed = true;
 		}
@@ -2339,6 +2495,48 @@ int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, 
 	if (pairs_changed) {
 		e->max_bus = *std::max_element(e->route_bus.begin(), e->route_bus.end());
 		e->bus_plan_dirty = true;
+	}
+	return OALSFX_OK;
+}
+}
+
+int oalsfx_engine_set_routes(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream, const int32_t* bus,
+	const float* gain, int ramp_frames)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	return set_routes_impl(e, first_stream, n_streams, routes_per_stream, bus, gain, nullptr, ramp_frames);
+}
+
+int oalsfx_engine_set_route_pans(oalsfx_engine* e, int first_stream, int n_streams, int routes_per_stream, const int32_t* bus,
+	const float* pan, int ramp_frames)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	if (!pan) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "Null pan matrices.");
+	}
+	return set_routes_impl(e, first_stream, n_streams, routes_per_stream, bus, nullptr, pan, ramp_frames);
+}
+
+int oalsfx_engine_set_bus_format(oalsfx_engine* e, int channel_format)
+{
+	if (!e) {
+		return OALSFX_ERR_ARGUMENT;
+	}
+	DeviceLayout d;
+	if (!make_device_layout(channel_format, d)) {
+		return e->fail(OALSFX_ERR_FORMAT, "Invalid channel format.");
+	}
+	if (d.channels != e->bus_channels && e->pan_routes > 0) {
+		return e->fail(OALSFX_ERR_ARGUMENT, "Pan routes are sized for the current bus channel count.");
+	}
+	e->quiesce();
+	if (d.channels != e->bus_channels) {
+		e->bus_channels = d.channels;
+		e->gains_dirty = true;   // the plan may change kernels: the gain image decides again whether it is needed
 	}
 	return OALSFX_OK;
 }

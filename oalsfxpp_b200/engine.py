@@ -71,6 +71,10 @@ def bind(lib):
     lib.oalsfx_engine_route_streams.restype = i32
     lib.oalsfx_engine_set_routes.argtypes = [vp, i32, i32, i32, vp, vp, i32]
     lib.oalsfx_engine_set_routes.restype = i32
+    lib.oalsfx_engine_set_bus_format.argtypes = [vp, i32]
+    lib.oalsfx_engine_set_bus_format.restype = i32
+    lib.oalsfx_engine_set_route_pans.argtypes = [vp, i32, i32, i32, vp, vp, i32]
+    lib.oalsfx_engine_set_route_pans.restype = i32
     lib.oalsfx_engine_reduce_buses.argtypes = [vp, i32, vp, i32, i32, vp, vp]
     lib.oalsfx_engine_reduce_buses.restype = i32
     lib.oalsfx_engine_mix_buses.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp]
@@ -119,7 +123,8 @@ def bind(lib):
 EXPORTED_SYMBOLS = (
     "oalsfx_engine_create", "oalsfx_engine_destroy", "oalsfx_engine_set_effect",
     "oalsfx_engine_set_sends", "oalsfx_engine_set_active", "oalsfx_engine_reset_streams", "oalsfx_engine_mix", "oalsfx_engine_mix_bus", "oalsfx_engine_reduce_bus",
-    "oalsfx_engine_route_streams", "oalsfx_engine_set_routes", "oalsfx_engine_reduce_buses", "oalsfx_engine_mix_buses",
+    "oalsfx_engine_route_streams", "oalsfx_engine_set_routes", "oalsfx_engine_set_bus_format",
+    "oalsfx_engine_set_route_pans", "oalsfx_engine_reduce_buses", "oalsfx_engine_mix_buses",
     "oalsfx_engine_pin_host", "oalsfx_engine_unpin_host",
     "oalsfx_engine_debug_state", "oalsfx_debug_waveshaper", "oalsfx_plan_placement", "oalsfx_engine_launch_count", "oalsfx_engine_last_kernel", "oalsfx_engine_device_bytes",
     "oalsfx_last_error", "oalsfx_build_info", "oalsfx_effect_defaults", "oalsfx_effect_normalize",
@@ -183,6 +188,7 @@ class Engine:
         self.channels = channel_count(channel_format)
         self.sampling_rate = int(sampling_rate)
         self.effect_count = int(effect_count)
+        self.bus_format = self.channel_format
         desc = _Desc(int(device), self.num_streams, self.channel_format, self.sampling_rate, self.effect_count)
         handle = C.c_void_p()
         rc = self.lib.oalsfx_engine_create(C.byref(desc), C.byref(handle))
@@ -304,16 +310,41 @@ class Engine:
         self._check(self.lib.oalsfx_engine_set_routes(self._h, int(first_stream), int(n), int(R), bus.ctypes.data,
                                                       None if g is None else g.ctypes.data, int(ramp_frames)))
 
+    def set_bus_format(self, channel_format):
+        """Every submix bus gets `channel_format` (a ChannelFormat; default: the engine's).  reduce_buses / mix_buses then
+        write [n_buses][frames][bus_channels].  Refused while a pan route exists and the channel count would change."""
+        self._check(self.lib.oalsfx_engine_set_bus_format(self._h, int(channel_format)))
+        self.bus_format = int(channel_format)
+
+    @property
+    def bus_channels(self):
+        """Channel count Cb of the submix buses."""
+        return channel_count(self.bus_format)
+
+    def set_route_pans(self, pan, bus, first_stream=0, ramp_frames=0):
+        """Pan routes of streams first_stream, first_stream + 1, ...: bus[i] as in set_routes, each route with a
+        [bus_channels][channels] matrix pan[i][r] (weight of stream channel k in bus channel j at [j][k]), its coefficients
+        ramped from the route's current ones over ramp_frames frames.  `pan` is [n][R][Cb][C] with `bus` [n][R], or
+        [n][Cb][C] with a 1-D `bus` (one route per stream)."""
+        bus = np.asarray(bus, dtype=np.int32)
+        if bus.ndim == 1:
+            bus = bus[:, None]
+        bus = np.ascontiguousarray(bus)
+        n, R = bus.shape
+        m = np.ascontiguousarray(np.asarray(pan, dtype=np.float32).reshape(n, R, self.bus_channels, self.channels))
+        self._check(self.lib.oalsfx_engine_set_route_pans(self._h, int(first_stream), int(n), int(R), bus.ctypes.data,
+                                                          m.ctypes.data, int(ramp_frames)))
+
     def _bus_count(self, frames, buses, n_buses):
         if n_buses is not None:
             return int(n_buses)
         size = buses.size if isinstance(buses, np.ndarray) else buses.numel() if hasattr(buses, "numel") else None
         if size is None:
             raise ValueError("n_buses is required for raw pointers")
-        return size // (int(frames) * self.channels)
+        return size // (int(frames) * self.bus_channels)
 
     def reduce_buses(self, frames, dst, buses, layout=LAYOUT_STREAM_MAJOR, stream=0, n_buses=None):
-        """buses ([n_buses][frames][channels], device) = per bus the sum of the rows of `dst` (device, as mix() wrote it) of
+        """buses ([n_buses][frames][bus_channels], device) = per bus the sum of the rows of `dst` (device, as mix() wrote it) of
         the active streams routed to it, in the fixed order of include/oalsfx_engine.h.  n_buses defaults to the size of
         `buses`."""
         self._check(self.lib.oalsfx_engine_reduce_buses(self._h, int(frames), _ptr(dst), layout,
